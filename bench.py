@@ -25,6 +25,13 @@ all-reduce). At N > 1 every config also verifies, outside the timed region, that
 the sum of the per-rank planes and that the counts cover N x the shard.
 
 `--impl reference` times only the CPU implementation of the headline config (all host threads).
+
+`--dump-outputs DIR` writes what the last timed step of the headline config computed on rank 0 as DIR/<name>.npy:
+per tiled decoder k the index, distance and confidence of a fixed, seeded sample of the reads (d<k>_*), the qcfail
+flags of the same reads, which reads they are (reads.npy), and every decoder's accumulator tables (d<k>_counts,
+d<k>_sums) and the chain totals. The synthetic inputs depend only on the arguments, so two builds run with the same
+arguments can be compared file for file: exactly, except the f64 confidence sums (d<k>_sums), which the kernels add
+atomically in no fixed order and so agree to rounding.
 """
 from __future__ import annotations
 
@@ -57,6 +64,11 @@ WORKLOAD_LABEL = {
 }
 NCU_SUMMARY = os.path.join(ROOT, "profiles", "ncu_summary.json")
 ORIGINAL_AFFINITY = None
+# --dump-outputs: per-read outputs of this many reads (drawn with DUMP_SEED), so that the files of the largest
+# configuration (c5: 47 MB of accumulator tables) stay under 64 MB in all
+DUMP_READS = 1 << 19
+DUMP_SEED = 20240601
+DUMP_LIMIT_BYTES = 64_000_000
 
 
 def algorithmic_bytes_per_read(chain, compiled) -> int:
@@ -271,10 +283,10 @@ class Bench:
         self.flush.zero_()
 
     # ------------------------------------------------------------------ one pass, timed
-    def timed_steps(self, chain, tiles, n, flags, results, steps, warmup, flush, warm_reads=None):
+    def timed_steps(self, chain, tiles, n, flags, results, steps, warmup, flush, warm_reads=None, capture=False):
         """`warmup` untimed steps (over the first warm_reads reads when given), then `steps` timed ones between barriers.
         Returns (elapsed ms max over ranks, clocks summary, launches inside the timed region, device ms of the last
-        timed step's kernels alone)."""
+        timed step's kernels alone, the last timed step's outputs when `capture` else None)."""
         torch = self.torch
 
         def step(m, collect=True):
@@ -301,6 +313,13 @@ class Bench:
             self.barrier()
             launches = chain.statistics()["kernel_launches"] - launches_before
             last_kernel_ms = chain.last_kernel_milliseconds()
+            outputs = None
+            if capture:
+                # read before anything below decodes again (over other reads for c5) or resets the accumulators; the copy
+                # leaves the GPU idle, so it stays out of the clock samples
+                clocks.end()
+                outputs = self.step_outputs(chain, n, flags, results)
+                clocks.begin()
             # keep the GPU under the same load a little longer when the timed region was too short to sample
             # (without the collective: every rank decides for itself how long it keeps going)
             extra = 0
@@ -312,7 +331,36 @@ class Bench:
                     torch.cuda.synchronize(self.device)
             torch.cuda.synchronize(self.device)
             clocks.end()
-        return self.max_over_ranks(start.elapsed_time(stop)), clocks.summary(), int(launches), last_kernel_ms
+        return self.max_over_ranks(start.elapsed_time(stop)), clocks.summary(), int(launches), last_kernel_ms, outputs
+
+    def step_outputs(self, chain, n, flags, results):
+        """What a caller of the timed path receives from one step, as float arrays for --dump-outputs: per-read results
+        and qcfail flags of DUMP_READS reads drawn with DUMP_SEED (all reads when fewer), every decoder's accumulator
+        tables and the chain totals."""
+        torch = self.torch
+        from pheniqs_b200 import RESULT_DTYPE
+        reads = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_READS), replace=False))
+        rows = torch.from_numpy(reads).to(self.device)
+        out = {"reads": reads.astype(np.float64), "qcfail": flags[rows].cpu().numpy().astype(np.float32)}
+        for k in range(chain.n_decoders):
+            if results[k] is not None:
+                record = results[k][rows].cpu().numpy().view(RESULT_DTYPE).reshape(-1)
+                out["d%d_index" % k] = record["index"].astype(np.float32)
+                out["d%d_distance" % k] = record["distance"].astype(np.float32)
+                out["d%d_confidence" % k] = record["confidence"].astype(np.float64)
+            u, f = chain.accumulators(k)
+            out["d%d_counts" % k] = u.astype(np.float64)
+            out["d%d_sums" % k] = f
+        out["totals"] = np.array(chain.totals(), dtype=np.float64)
+        return out
+
+    @staticmethod
+    def dump_bytes(chain, n):
+        """The bytes step_outputs returns for this chain and batch, known before anything runs."""
+        sampled = min(n, DUMP_READS)
+        per_read = 8 + 4 + sum(4 + 4 + 8 for info in chain.info if info.has_tile)
+        tables = sum((info.barcode_cardinality + 1) * (6 + 2) * 8 for info in chain.info)
+        return sampled * per_read + tables + 2 * 8
 
     def kernel_only(self, chain, tiles, n, flags, results, repeats):
         """The decoders' kernels alone (no reset, flush or collective), CUDA events on the launching stream."""
@@ -426,8 +474,11 @@ class Bench:
         bytes_per_read = algorithmic_bytes_per_read(chain, compiled)
         # timing rule: inputs larger than L2, or L2 flushed between steps (a 256 MB write inside the step)
         flush = bytes_per_read * n < (192 << 20)
+        capture = headline and self.args.dump_outputs is not None and self.rank == 0
+        if capture and self.dump_bytes(chain, n) > DUMP_LIMIT_BYTES:
+            raise SystemExit("bench.py: --dump-outputs would write %d bytes, more than %d" % (self.dump_bytes(chain, n), DUMP_LIMIT_BYTES))
 
-        elapsed_ms, clocks, launches, last_kernel_ms = self.timed_steps(chain, tiles, n, flags, results, steps, warmup, flush, warm_reads)
+        elapsed_ms, clocks, launches, last_kernel_ms, outputs = self.timed_steps(chain, tiles, n, flags, results, steps, warmup, flush, warm_reads, capture)
         # the kernels alone: a few more passes, or (long single-step configs) the events of the timed step itself
         kernel_ms = self.kernel_only(chain, tiles, n, flags, results, min(steps, 5)) if steps >= 3 else last_kernel_ms
         collect_ms = self.collect_only(chain)
@@ -448,7 +499,7 @@ class Bench:
             entry["two_pass"] = self.two_pass(chain, compiled, spec, tiles, n, flags, results, steps, warmup, flush, sampling)
         if self.rank == 0 and self.world == 1 and not self.args.no_cpu_baseline:
             entry["cpu_baseline"] = time_cpu(compiled, spec, seconds_target=12.0 if headline else 4.0)
-        return entry, (spec, compiled, chain, tiles)
+        return entry, (spec, compiled, chain, tiles, outputs)
 
     def two_pass(self, chain, compiled, spec, tiles, n, flags, results, steps, warmup, flush, sampling):
         """The two-pass workflow (docs/pamld.md:38-44; C4 names it): pass 1 under the configured (uniform) priors -> collect (NCCL) ->
@@ -490,7 +541,7 @@ class Bench:
         stage["kernels_pass2"] = "; ".join(chain.kernel_description(k) for k in range(chain.n_decoders))
 
         # pass 2 as a timed run of its own, same rules as pass 1
-        elapsed_ms, clocks, launches, _ = self.timed_steps(chain, tiles, n, flags, results, steps, warmup, flush)
+        elapsed_ms, clocks, launches, _, _ = self.timed_steps(chain, tiles, n, flags, results, steps, warmup, flush)
         kernel_ms = self.kernel_only(chain, tiles, n, flags, results, min(steps, 5))
         stage["pass2"] = {"value": n * self.world * steps / (elapsed_ms * 1e-3), "unit": UNIT, "ms_per_step": elapsed_ms / steps, "steps": steps,
                           "roofline": self.roofline("c4_pass2", chain, compiled, n, kernel_ms, clocks), "gpu_launches": launches, "clocks": clocks}
@@ -700,7 +751,13 @@ def main():
     parser.add_argument("--impl", default="b200", choices=["b200", "reference"])
     parser.add_argument("--no-cpu-baseline", action="store_true")
     parser.add_argument("--no-e2e", action="store_true")
+    parser.add_argument("--dump-outputs", metavar="DIR", default=None,
+                        help="write what the last timed step of the headline configuration computed as DIR/<name>.npy")
     args = parser.parse_args()
+    if args.steps < 1:
+        parser.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        parser.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -724,7 +781,12 @@ def main():
     bench = Bench(args, rank, local_rank, world)
     n = args.reads or DEFAULT_READS[args.workload]
     warm_reads = SHORT_RUN["c5"][1] if args.workload == "c5" else None
-    entry, (spec, compiled, chain, tiles) = bench.run(args.workload, n, args.steps, args.warmup, warm_reads=warm_reads, headline=True)
+    entry, (spec, compiled, chain, tiles, outputs) = bench.run(args.workload, n, args.steps, args.warmup, warm_reads=warm_reads, headline=True)
+    if outputs is not None and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, array in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), array)
+    del outputs
     line = {"metric": METRIC, "value": entry["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": entry["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f64", "data": "synthetic",
@@ -744,7 +806,7 @@ def main():
     for name in [c for c in args.configs.split(",") if c and c != args.workload]:
         reads, warm, steps = SHORT_RUN[name]
         try:
-            entry, (spec_k, compiled_k, chain, tiles) = bench.run(name, reads, steps, 3, warm_reads=warm)
+            entry, (spec_k, compiled_k, chain, tiles, _) = bench.run(name, reads, steps, 3, warm_reads=warm)
             if not args.no_e2e:
                 bench.end_to_end(entry, spec_k, compiled_k, chain, tiles, reads, brief=True, brief_reads=(1 << 22) if name == "c5" else (1 << 24))
             configs[name] = entry

@@ -1,4 +1,5 @@
 import os
+import subprocess
 import sys
 
 import pytest
@@ -39,6 +40,7 @@ def built():
     from oracle import oracle
     if not os.path.exists(oracle.PORT_LIBRARY):
         oracle.build("port")
-    if not oracle.ref_available() and os.path.exists("/root/reference/pamld.cpp"):
-        oracle.build("ref")
+    reference = os.environ.get("PHENIQS_REFERENCE")         # the upstream Pheniqs sources, to build oracle/_ref from
+    if not oracle.ref_available() and reference and os.path.exists(os.path.join(reference, "pamld.cpp")):
+        subprocess.run(["make", "-s", "-C", oracle.HERE, "ref", "REFERENCE=" + reference], check=True)
     return True

@@ -1,8 +1,12 @@
 """The C restatement against the reference's own classes (oracle/_ref) on seeded synthetic reads.
 
 MDD, multi-segment PAMLD, reverse complement knits and barcode counts above 5 have no stored vector in the
-reference's tests (SURVEY.md §8c); here the restatement is pinned on them by the live reference build.
-Skipped where oracle/_ref could not be built (needs /root/reference at build time)."""
+reference's tests (SURVEY.md §8c); here the restatement is pinned on them by the live reference build where oracle/_ref
+is built, and everywhere by tests/golden/reference_outputs.json: a SHA-256 of every array compared below
+(tests/golden/make_reference_vectors.py; its "source" names the checker that computed them)."""
+import hashlib
+import zlib
+
 import numpy as np
 import pytest
 
@@ -10,44 +14,55 @@ import helpers
 from oracle import oracle as O
 from pheniqs_b200 import workload
 
-pytestmark = pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref not built")
+VARIANTS = ["pamld", "pamld_hq", "pamld_rc2", "mdd", "mdd_masked", "mdd_rc"]
 
 
-def both(compiled, batch, n_segments):
-    port, ref = O.PortOracle(compiled), O.RefOracle(compiled, n_segments)
-    a, b = port.decode(batch), ref.decode(batch)
-    assert np.array_equal(a.index, b.index)
-    assert np.array_equal(a.distance, b.distance)
-    assert np.array_equal(a.confidence, b.confidence)          # same operation order -> bit identical
-    assert np.array_equal(a.qcfail, b.qcfail)
-    assert np.array_equal(a.read_distance, b.read_distance)
-    assert np.array_equal(a.read_confidence, b.read_confidence)
-    assert np.array_equal(a.channel, b.channel)
-    for k in range(port.n_decoders):
-        ua, fa = port.accumulators(k)
-        ub, fb = ref.accumulators(k)
-        assert np.array_equal(ua, ub) and np.array_equal(fa, fb)
-        if port.chain[k][1]["algorithm"] == "pamld":
-            na, ca = port.estimate_priors(k)
-            nb, cb = ref.estimate_priors(k)
-            assert na == nb and np.array_equal(ca, cb)
-    assert port.totals() == ref.totals()
-    return a
+def outputs(oracle, batch):
+    """Everything a checker reports for one batch, by name: per-read results, accumulators, estimated priors, totals."""
+    out = oracle.decode(batch)
+    arrays = {name: getattr(out, name) for name in ("index", "distance", "confidence", "qcfail", "read_distance", "read_confidence", "channel")}
+    for k in range(oracle.n_decoders):
+        arrays["counts%d" % k], arrays["sums%d" % k] = oracle.accumulators(k)
+        if oracle.chain[k][1]["algorithm"] == "pamld":
+            noise, concentration = oracle.estimate_priors(k)
+            arrays["noise%d" % k] = np.array([noise], dtype=np.float64)
+            arrays["concentration%d" % k] = concentration
+    arrays["totals"] = np.array(oracle.totals(), dtype=np.uint64)
+    return arrays
 
 
-@pytest.mark.parametrize("name", ["c1", "c2", "c3", "c4"])
-def test_baseline_configs(name):
+def digests(arrays):
+    """SHA-256 of each array's dtype, shape and bytes: equal digests = bit identical arrays."""
+    out = {}
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a)
+        out[name] = hashlib.sha256(("%s %s " % (a.dtype.str, a.shape)).encode() + a.tobytes()).hexdigest()
+    return out
+
+
+def both(case, compiled, batch, n_segments):
+    port = outputs(O.PortOracle(compiled), batch)
+    stored = helpers.golden("reference_outputs.json")[case]
+    got = digests(port)
+    assert sorted(got) == sorted(stored), case
+    assert [name for name in stored if got[name] != stored[name]] == [], case + ": differs from the stored outputs"
+    if O.ref_available():
+        ref = outputs(O.RefOracle(compiled, n_segments), batch)
+        assert sorted(ref) == sorted(port)
+        for name in port:
+            assert np.array_equal(port[name], ref[name]), case + " " + name          # same operation order -> bit identical
+    return port
+
+
+def baseline_inputs(name):
     spec = workload.load(name)
     compiled = O.compile_job(spec["job"])
     code, quality, offset, _ = workload.synthesize(compiled, spec["input segment length"], 3000, seed=11)
-    out = both(compiled, O.ReadBatch(code, quality, offset), len(code))
-    assert (out.index > 0).any()
+    return compiled, O.ReadBatch(code, quality, offset), len(code)
 
 
-@pytest.mark.parametrize("short", [0.0, 0.2])
-@pytest.mark.parametrize("variant", ["pamld", "pamld_hq", "pamld_rc2", "mdd", "mdd_masked", "mdd_rc"])
-def test_random_decoders(variant, short):
-    rng = np.random.default_rng(hash(variant) % 1000)
+def random_inputs(variant, short):
+    rng = np.random.default_rng(zlib.crc32(variant.encode()) % 1000)
     if variant == "pamld":
         decoder = helpers.random_job(rng, "pamld", (8,), 24)
     elif variant == "pamld_hq":
@@ -67,12 +82,10 @@ def test_random_decoders(variant, short):
     compiled = O.compile_job(job)
     code, quality, offset, _ = workload.synthesize(compiled, [0], 2500, seed=5, short_fraction=short)
     qcfail = (rng.random(2500) < 0.1).astype(np.uint8)
-    out = both(compiled, O.ReadBatch(code, quality, offset, qcfail), len(code))
-    assert out.qcfail.sum() >= qcfail.sum()
+    return compiled, O.ReadBatch(code, quality, offset, qcfail), len(code)
 
 
-def test_degenerate_observations():
-    """all-N, all-Q0 and all-Q2 observations: the noise filter and the first-maximum rule on exact ties."""
+def degenerate_inputs():
     rng = np.random.default_rng(3)
     job = {"sample": helpers.random_job(rng, "pamld", (8,), 10)}
     for record in job["sample"]["codec"].values():
@@ -87,15 +100,48 @@ def test_degenerate_observations():
     quality[32:48] = 2
     code[48:] = np.array([1, 2, 4, 8, 1, 2, 4, 8, 1, 2], dtype=np.uint8)
     quality[48:] = rng.integers(0, 42, size=(16, 10))
-    batch = O.ReadBatch.from_fixed([code], [quality])
-    both(compiled, batch, 1)
+    return compiled, O.ReadBatch.from_fixed([code], [quality]), 1
+
+
+def whitelist_inputs():
+    spec = workload.load("c5", whitelist_cardinality=4000)
+    compiled = O.compile_job(spec["job"])
+    code, quality, offset, _ = workload.synthesize(compiled, spec["input segment length"], 400, seed=5)
+    return compiled, O.ReadBatch(code, quality, offset), len(code)
+
+
+def cases():
+    """(key in reference_outputs.json, inputs) of every test below."""
+    for name in ("c1", "c2", "c3", "c4"):
+        yield "baseline_" + name, lambda name=name: baseline_inputs(name)
+    for variant in VARIANTS:
+        for short in (0.0, 0.2):
+            yield "random_%s_%g" % (variant, short), lambda variant=variant, short=short: random_inputs(variant, short)
+    yield "degenerate", degenerate_inputs
+    yield "whitelist_reduced", whitelist_inputs
+
+
+@pytest.mark.parametrize("name", ["c1", "c2", "c3", "c4"])
+def test_baseline_configs(name):
+    out = both("baseline_" + name, *baseline_inputs(name))
+    assert (out["index"] > 0).any()
+
+
+@pytest.mark.parametrize("short", [0.0, 0.2])
+@pytest.mark.parametrize("variant", VARIANTS)
+def test_random_decoders(variant, short):
+    compiled, batch, n_segments = random_inputs(variant, short)
+    out = both("random_%s_%g" % (variant, short), compiled, batch, n_segments)
+    assert out["qcfail"].sum() >= batch.qcfail.sum()
+
+
+def test_degenerate_observations():
+    """all-N, all-Q0 and all-Q2 observations: the noise filter and the first-maximum rule on exact ties."""
+    both("degenerate", *degenerate_inputs())
 
 
 def test_whitelist_config_reduced():
     """Config 5's shape (16 nt cellular whitelist + naive UMI) on 4,000 barcodes: the restatement and the reference's own
     classes agree bit for bit there too (the full 737,280 barcode table is covered on the GPU box against oracle/_ref)."""
-    spec = workload.load("c5", whitelist_cardinality=4000)
-    compiled = O.compile_job(spec["job"])
-    code, quality, offset, _ = workload.synthesize(compiled, spec["input segment length"], 400, seed=5)
-    out = both(compiled, O.ReadBatch(code, quality, offset), len(code))
-    assert (out.index > 0).any()
+    out = both("whitelist_reduced", *whitelist_inputs())
+    assert (out["index"] > 0).any()
