@@ -956,9 +956,9 @@ int phq_pack(phq_handle* handle, int64_t n_reads, int32_t n_input_segments,
                         for(int32_t i(0); i < d.segment_length[sgm]; ++i) {
                             const int32_t j(d.segment_offset[sgm] + i);
                             if(!stale_semantics && i >= from.length) {
-                                /* Sequence::distance_from stops at the observed length: the position is absent, marked by
-                                   PHQ_ABSENT_QUALITY and, so that kernels that never read qualities see it too, by an
-                                   ambiguous position whose base bits are both set (a real ambiguous base has them clear) */
+                                /* Sequence::distance_from stops at the observed length: the position is absent, marked as
+                                   an ambiguous position whose base bits are both set (a real ambiguous base has them clear),
+                                   quality PHQ_ABSENT_QUALITY */
                                 phred[j] = PHQ_ABSENT_QUALITY;
                                 lo |= 1u << j;
                                 hi |= 1u << j;

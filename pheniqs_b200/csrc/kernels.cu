@@ -153,6 +153,12 @@ __device__ __forceinline__ uint32_t quality_word(const TileArguments& A, long lo
     return 0u;
 }
 
+/*  The row of the 128-entry Phred tables a quality byte scores with. The reference's tables end at 127 and a byte
+    above (a FASTQ decoded at too high an offset, a BAM record without qualities) indexes past them; such a byte
+    carries no information and scores 0, as q = 0 does (DESIGN.md §5). The high quality filter still compares
+    the raw byte. */
+__device__ __forceinline__ uint32_t phred_quality(uint32_t q) { return q > 127u ? 0u : q; }
+
 /* ------------------------------------------------------------------ per-CTA accumulators
    AccumulatingOption (selector.h:32-60). Staged in shared memory (u32 counters, f64 sums) when the
    table is small, flushed with one global atomic per non-zero cell; straight to global otherwise. */
@@ -229,11 +235,12 @@ __device__ __forceinline__ BlockState block_prologue(unsigned char* smem, const 
         for(int i = tid; i < 256; i += blockDim.x) { s.phred[i] = P.phred[i]; }
     }
     if(ratio32) {
-        /* what one position contributes, by Phred byte (0..255, clamped at 127 like the reference's table) and,
-           from entry 256 on, for a base that is not A / C / G / T: one 16-byte load per position */
+        /* what one position contributes, by Phred byte (0..255; a byte above 127 carries no information and scores as
+           q = 0: phred_quality) and, from entry 256 on, for a base that is not A / C / G / T: one 16-byte load
+           per position */
         PositionEntry* const position = reinterpret_cast< PositionEntry* >(smem + s.plan.off_ratio32);
         for(int i = tid; i < 512; i += blockDim.x) {
-            const int q = (i & 255) > 127 ? 127 : (i & 255);
+            const int q = static_cast< int >(phred_quality(static_cast< uint32_t >(i & 255)));
             PositionEntry e;
             e.pad = 0u;
             if(i < 256) {
@@ -603,7 +610,7 @@ struct PositionFactor {
 };
 __device__ __forceinline__ PositionFactor position_factor(const double* __restrict__ phred_shared, double uniform_factor, uint32_t q, bool ambiguous) {
     PositionFactor f;
-    q = q > 127u ? 127u : q;
+    q = phred_quality(q);
     f.factor = phred_shared[PHRED_MATCH_FACTOR + q];
     f.ratio = phred_shared[PHRED_MISMATCH_RATIO + q];
     f.uniform = ambiguous && q != 0u;
@@ -1256,8 +1263,7 @@ __device__ __forceinline__ double exact_product(const double* __restrict__ ratio
         uint32_t word = quality[0];
         #pragma unroll
         for(int g = 1; g < G; ++g) { if((j >> 2) == g) { word = quality[g]; } }
-        uint32_t q = (word >> (8 * (j & 3))) & 0xffu;
-        q = q > 127u ? 127u : q;
+        const uint32_t q = phred_quality((word >> (8 * (j & 3))) & 0xffu);
         t *= ratio64[q];
     }
     return t;
@@ -2499,8 +2505,7 @@ pamld_tie_kernel(const DecoderParams P, const TileArguments A) {
         uint32_t score_address[4 * G];
         #pragma unroll
         for(int j = 0; j < 4 * G; ++j) {
-            uint32_t q = (record.quality[j >> 2] >> (8 * (j & 3))) & 0xffu;
-            q = q > 127u ? 127u : q;
+            const uint32_t q = phred_quality((record.quality[j >> 2] >> (8 * (j & 3))) & 0xffu);
             score_address[j] = score_table + q * 8u + ((nmask >> j) & 1u) * 2048u;
         }
 
@@ -2681,19 +2686,19 @@ mdd_kernel(const DecoderParams P, const TileArguments A) {
                 o_hi |= w1 & 0xffff0000u;
                 nmask |= load_stream(A.nmask + A.pitch + r) << 16;
             }
-            for(int g = 0; g < P.quality_word_cardinality; ++g) {
-                const uint32_t qw = quality_word(A, r, g);
-                #pragma unroll
-                for(int k = 0; k < 4; ++k) {
-                    const uint32_t q = (qw >> (8 * k)) & 0xffu;
-                    const int j = g * 4 + k;
-                    if(q != PHQ_ABSENT_QUALITY) { present |= 1u << j; }
-                    if(static_cast< int >(q) < P.quality_masking_threshold) { masked |= 1u << j; }
+            /* a position the read does not have is packed as ambiguous with both base bits set (a real ambiguous base
+               has them clear); the quality byte is a Phred value like any other, 255 included */
+            present = ~(nmask & o_lo & o_hi) & all_positions;
+            if(P.quality_masking_threshold > 0) {
+                for(int g = 0; g < P.quality_word_cardinality; ++g) {
+                    const uint32_t qw = quality_word(A, r, g);
+                    #pragma unroll
+                    for(int k = 0; k < 4; ++k) {
+                        if(static_cast< int >((qw >> (8 * k)) & 0xffu) < P.quality_masking_threshold) { masked |= 1u << (g * 4 + k); }
+                    }
                 }
+                masked &= present;
             }
-            present &= all_positions;
-            masked &= present;
-            if(P.quality_masking_threshold <= 0) { masked = 0; }
             qcfail = A.qcfail[r];
         }
         const bool complete = present == all_positions;
