@@ -32,7 +32,9 @@ extern "C" {
 
 #define PHQ_VERSION "0.1.0"
 #define PHQ_MAX_SEGMENTS 8          /* output segments of one decoder's Observation */
-#define PHQ_MAX_NUCLEOTIDES 32      /* nucleotide cardinality of one decoder (two 16-base words) */
+#define PHQ_MAX_NUCLEOTIDES 64      /* nucleotide cardinality of one decoder (four 16-base words); no struct of this
+                                       header is sized by it. Decoders of more than 32 run on kernels of their own
+                                       and cannot use the compact result forms above 63 (a 6-bit distance) */
 #define PHQ_ABSENT_QUALITY 0xFF     /* quality byte phq_pack writes at a position the (short) read does not have; the
                                        kernels recognise such a position by its planes (phq_tile), not by this byte */
 

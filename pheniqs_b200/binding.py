@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIBRARY_PATH = os.path.join(HERE, "libpheniqs_b200.so")
 
 PHQ_MAX_SEGMENTS = 8
-PHQ_MAX_NUCLEOTIDES = 32
+PHQ_MAX_NUCLEOTIDES = 64
 PHQ_ABSENT_QUALITY = 0xFF
 
 PHQ_OK = 0

@@ -98,6 +98,7 @@ struct phq_handle {
     std::vector< DecoderParams > params;
     std::vector< std::vector< ScratchSegment > > scratch;
     std::vector< BarcodeEntry* > device_barcodes;
+    std::vector< LongBarcodeEntry* > device_long;   /* the table of decoders of more than LONG_NUCLEOTIDES (kernels.cuh), NULL elsewhere */
     std::vector< MddSlot* > device_mdd;        /* MDD lookup tables (kernels.cuh), NULL where the scan kernel is used */
     std::vector< std::vector< int32_t > > mdd_shape;    /* per decoder: first slot and mask of every table, total slots */
     std::vector< uint8_t* > device_barcode_code;   /* tag synthesis: [(N + 1)][L] BAM codes per coded decoder, row 0 undetermined */
@@ -172,6 +173,30 @@ void assemble_phred(std::vector< double >& table, double& uniform_quality, doubl
 
 void upload_barcodes(phq_handle* h, size_t k) {
     const DecoderSpec& d(h->chain[k]);
+    if(d.nucleotide_cardinality > LONG_NUCLEOTIDES) {
+        /* split form: positions [0, split) in the first word of each plane, [split, L) in the second */
+        const int32_t split(long_split(d.nucleotide_cardinality));
+        std::vector< LongBarcodeEntry > table(static_cast< size_t >(d.barcode_cardinality));
+        for(int32_t b(0); b < d.barcode_cardinality; ++b) {
+            LongBarcodeEntry e;
+            memset(&e, 0, sizeof(e));
+            for(int32_t j(0); j < d.nucleotide_cardinality; ++j) {
+                const uint8_t code(d.barcode[static_cast< size_t >(b) * d.nucleotide_cardinality + j]);
+                const uint32_t two(code == 1 ? 0u : code == 2 ? 1u : code == 4 ? 2u : 3u);
+                if(j < split) {
+                    e.lo0 |= (two & 1u) << j;
+                    e.hi0 |= (two >> 1) << j;
+                } else {
+                    e.lo1 |= (two & 1u) << (j - split);
+                    e.hi1 |= (two >> 1) << (j - split);
+                }
+            }
+            e.prior = d.concentration[b];
+            table[b] = e;
+        }
+        PHQ_CUDA(cudaMemcpy(h->device_long[k], table.data(), table.size() * sizeof(LongBarcodeEntry), cudaMemcpyHostToDevice));
+        return;
+    }
     std::vector< BarcodeEntry > table(static_cast< size_t >(d.barcode_cardinality));
     for(int32_t b(0); b < d.barcode_cardinality; ++b) {
         BarcodeEntry e;
@@ -192,7 +217,9 @@ void upload_barcodes(phq_handle* h, size_t k) {
 void upload_fast(phq_handle* h, size_t k) {
     const DecoderSpec& d(h->chain[k]);
     if(h->device_fast[k] != NULL) { cudaFree(h->device_fast[k]); h->device_fast[k] = NULL; }
-    if(d.algorithm != PHQ_PAMLD || !h->fast_enabled) { return; }
+    /* no prefilter for long decoders: its f32 error bound is argued for at most 32 positions, and 4^-64 is below the
+       smallest normal float */
+    if(d.algorithm != PHQ_PAMLD || !h->fast_enabled || d.nucleotide_cardinality > LONG_NUCLEOTIDES) { return; }
     std::vector< FastEntry > table(static_cast< size_t >(d.barcode_cardinality));
     for(int32_t b(0); b < d.barcode_cardinality; ++b) {
         FastEntry e;
@@ -361,6 +388,7 @@ void upload_mdd_tables(phq_handle* h, size_t k) {
     if(h->device_mdd[k] != NULL) { cudaFree(h->device_mdd[k]); h->device_mdd[k] = NULL; }
     h->mdd_shape[k].clear();
     if(d.algorithm != PHQ_MDD || d.segment_cardinality > 4 || d.barcode_cardinality > MDD_MAX_BARCODES) { return; }
+    if(d.nucleotide_cardinality > LONG_NUCLEOTIDES) { return; }        /* the lookup kernel reads 32-position planes */
     const int32_t S(d.segment_cardinality);
     const int32_t L(d.nucleotide_cardinality);
     std::vector< std::vector< std::vector< uint8_t > > > words(static_cast< size_t >(S));      /* distinct words per segment, 2-bit codes */
@@ -482,10 +510,14 @@ void refresh_params(phq_handle* h, size_t k) {
     p.quality_word_cardinality = d.quality_word_cardinality();
     p.group_cardinality = d.quality_word_cardinality();
     p.segment_cardinality = d.segment_cardinality;
+    const bool long_form(d.nucleotide_cardinality > LONG_NUCLEOTIDES);
+    p.long_split = long_form ? long_split(d.nucleotide_cardinality) : 0;
     for(int32_t s(0); s < d.segment_cardinality && s < PHQ_MAX_SEGMENTS; ++s) {
-        uint32_t mask(0);
-        for(int32_t j(d.segment_offset[s]); j < d.segment_offset[s + 1]; ++j) { mask |= 1u << j; }
-        p.segment_mask[s] = mask;
+        /* long decoders: the mask in split form (kernels.cuh), word 0 here and word 1 in segment_mask_long */
+        uint64_t mask(0);
+        for(int32_t j(d.segment_offset[s]); j < d.segment_offset[s + 1]; ++j) { mask |= static_cast< uint64_t >(1) << j; }
+        p.segment_mask[s] = static_cast< uint32_t >(long_form ? (mask & ((static_cast< uint64_t >(1) << p.long_split) - 1)) : mask);
+        p.segment_mask_long[s] = long_form ? static_cast< uint32_t >(mask >> p.long_split) : 0u;
         p.distance_tolerance[s] = d.algorithm == PHQ_MDD ? d.distance_tolerance[s] : 0;
     }
     p.high_quality_threshold = d.high_quality_threshold;
@@ -507,6 +539,7 @@ void refresh_params(phq_handle* h, size_t k) {
         p.uniform_observation_probability = pow(pow(10.0, -0.1), sigma);
     }
     p.barcodes = h->device_barcodes[k];
+    p.long_barcodes = h->device_long[k];
     p.phred = h->device_phred;
     p.acc_u64 = h->u64_plane() + h->offset_u64[k];
     p.acc_f64 = h->f64_plane() + h->offset_f64[k];
@@ -557,6 +590,7 @@ void destroy(phq_handle* h) {
     if(h->device < 0) { delete h; return; }
     cudaSetDevice(h->device);
     for(auto* p : h->device_barcodes) { if(p != NULL) { cudaFree(p); } }
+    for(auto* p : h->device_long) { if(p != NULL) { cudaFree(p); } }
     for(auto* p : h->device_grid) { if(p != NULL) { cudaFree(p); } }
     for(auto* p : h->device_fast) { if(p != NULL) { cudaFree(p); } }
     if(h->device_phred32 != NULL) { cudaFree(h->device_phred32); }
@@ -696,11 +730,14 @@ template < class F > int guarded(phq_handle* h, F body) {
 void refuse_collected(const phq_handle* h) {
     if(h->collected) { throw InternalError("the accumulators of this handle were collected across ranks; phq_reset_accumulators before the next pass"); }
 }
-/* phq_compact_result carries the barcode index in 24 bits */
+/* phq_compact_result carries the barcode index in 24 bits and the distance in 6 */
 void require_compact_range(const phq_handle* h) {
     for(const auto& d : h->chain) {
         if(d.tiled() && d.barcode_cardinality >= 0xffffff) {
             throw ConfigurationError("a decoder with " + std::to_string(d.barcode_cardinality) + " barcodes does not fit the 24 bit index of phq_compact_result; use the phq_result forms");
+        }
+        if(d.tiled() && d.nucleotide_cardinality > 63) {
+            throw ConfigurationError("a decoder of " + std::to_string(d.nucleotide_cardinality) + " nucleotides does not fit the 6 bit distance of phq_compact_result; use the phq_result forms");
         }
     }
 }
@@ -804,6 +841,7 @@ int phq_create(const char* compiled_job_json, int device, phq_handle** handle) {
         const size_t n(chain.size());
         h->params.resize(n);
         h->device_barcodes.assign(n, NULL);
+        h->device_long.assign(n, NULL);
         h->device_grid.assign(n, NULL);
         h->device_fast.assign(n, NULL);
         h->device_whitelist.assign(n, NULL);
@@ -842,10 +880,14 @@ int phq_create(const char* compiled_job_json, int device, phq_handle** handle) {
 
         for(size_t k(0); k < n; ++k) {
             if(chain[k].tiled()) {
-                /* padded to whole whitelist groups with zero entries (prior 0): pamld_whitelist_kernel may look a padding barcode up */
-                const size_t padded((static_cast< size_t >(chain[k].barcode_cardinality) + WHITELIST_CHUNK - 1) / WHITELIST_CHUNK * WHITELIST_CHUNK);
-                PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_barcodes[k]), padded * sizeof(BarcodeEntry)));
-                PHQ_CUDA(cudaMemset(h->device_barcodes[k], 0, padded * sizeof(BarcodeEntry)));
+                if(chain[k].nucleotide_cardinality > LONG_NUCLEOTIDES) {
+                    PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_long[k]), static_cast< size_t >(chain[k].barcode_cardinality) * sizeof(LongBarcodeEntry)));
+                } else {
+                    /* padded to whole whitelist groups with zero entries (prior 0): pamld_whitelist_kernel may look a padding barcode up */
+                    const size_t padded((static_cast< size_t >(chain[k].barcode_cardinality) + WHITELIST_CHUNK - 1) / WHITELIST_CHUNK * WHITELIST_CHUNK);
+                    PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_barcodes[k]), padded * sizeof(BarcodeEntry)));
+                    PHQ_CUDA(cudaMemset(h->device_barcodes[k], 0, padded * sizeof(BarcodeEntry)));
+                }
                 upload_barcodes(h, k);
                 upload_fast(h, k);
                 upload_grid(h, k);
@@ -947,7 +989,7 @@ int phq_pack(phq_handle* handle, int64_t n_reads, int32_t n_input_segments,
                         }
                     }
                     /* 2-bit planes + ambiguity mask + Phred bytes */
-                    uint32_t lo(0), hi(0), ambiguous(0);
+                    uint64_t lo(0), hi(0), ambiguous(0);
                     uint8_t phred[PHQ_MAX_NUCLEOTIDES];
                     memset(phred, 0, sizeof(phred));
                     for(int32_t sgm(0); sgm < d.segment_cardinality; ++sgm) {
@@ -960,25 +1002,26 @@ int phq_pack(phq_handle* handle, int64_t n_reads, int32_t n_input_segments,
                                    an ambiguous position whose base bits are both set (a real ambiguous base has them clear),
                                    quality PHQ_ABSENT_QUALITY */
                                 phred[j] = PHQ_ABSENT_QUALITY;
-                                lo |= 1u << j;
-                                hi |= 1u << j;
-                                ambiguous |= 1u << j;
+                                lo |= static_cast< uint64_t >(1) << j;
+                                hi |= static_cast< uint64_t >(1) << j;
+                                ambiguous |= static_cast< uint64_t >(1) << j;
                                 continue;
                             }
                             /* PAMLD reads the expected length: terminator, then stale bytes (barcode.h:150) */
                             const uint8_t c(from.code[i]);
+                            const uint64_t bit(static_cast< uint64_t >(1) << j);
                             switch(c) {
                                 case 1: break;
-                                case 2: lo |= 1u << j; break;
-                                case 4: hi |= 1u << j; break;
-                                case 8: lo |= 1u << j; hi |= 1u << j; break;
-                                default: ambiguous |= 1u << j; break;
+                                case 2: lo |= bit; break;
+                                case 4: hi |= bit; break;
+                                case 8: lo |= bit; hi |= bit; break;
+                                default: ambiguous |= bit; break;
                             }
                             phred[j] = from.quality[i];
                         }
                     }
                     for(int32_t w(0); w < words; ++w) {
-                        out_bases[w * pitch + r] = ((lo >> (16 * w)) & 0xffffu) | (((hi >> (16 * w)) & 0xffffu) << 16);
+                        out_bases[w * pitch + r] = static_cast< uint32_t >((lo >> (16 * w)) & 0xffffu) | (static_cast< uint32_t >((hi >> (16 * w)) & 0xffffu) << 16);
                         out_nmask[w * pitch + r] = static_cast< uint16_t >((ambiguous >> (16 * w)) & 0xffffu);
                     }
                     for(int32_t w(0); w < quality_words; ++w) {

@@ -6,6 +6,8 @@
     mdd_kernel     MdDecoder::classify (mdd.cpp:37-86) with Sequence::distance_from /
                    ObservedSequence::masked_distance_from (sequence.h:90-98, 321-332).
     count_kernel   the bookkeeping NaiveMolecularDecoder / passthrough classifiers do (naive.h:40-45).
+    pamld_long_kernel, pamld_long_tie_kernel, mdd_long_kernel
+                   the same for decoders of 33-64 nucleotides, over the split form of LongBarcodeEntry (kernels.cuh).
 
     Design (DESIGN.md has the long form). One lane owns one read; the barcode table streams
     through shared memory in 16 KB chunks moved by TMA bulk copies (cp.async.bulk + mbarrier),
@@ -548,15 +550,14 @@ constexpr double WHITELIST_BAND = 4.76837158203125e-07;      /* = WHITELIST_TOLE
    GUARDED: the caller has already kept the confidence away from its threshold (the prefilter scans' 2^-38 guard is
    wider than the diagnostic's band), so only the other threshold is watched */
 template < bool GUARDED = false >
-__device__ __forceinline__ Verdict pamld_apply(const DecoderParams& P, const Accumulator& accumulator, uint32_t* band_counter,
-                                               int best_index, uint32_t m, double conditional_probability, double confidence,
-                                               bool uniform, uint32_t high_quality_mask, uint32_t qcfail) {
+__device__ __forceinline__ Verdict pamld_apply_counted(const DecoderParams& P, const Accumulator& accumulator, uint32_t* band_counter,
+                                                       int best_index, int distance, int high_quality_distance, double conditional_probability,
+                                                       double confidence, bool uniform, uint32_t qcfail) {
     Verdict v;
     v.confidence = confidence;
-    v.distance = __popc(m);
+    v.distance = distance;
     v.decoded = best_index + 1;
     v.qcfail = qcfail;
-    const int high_quality_distance = __popc(m & high_quality_mask);
     const int best_row = best_index + 1;
 
     /* diagnostic: reads whose decision sits within the accuracy of this path of a threshold. 1e-12 for the exact and
@@ -590,16 +591,30 @@ __device__ __forceinline__ Verdict pamld_apply(const DecoderParams& P, const Acc
     accumulator.add_pair(v.decoded, ACC_COUNT, ACC_PF_COUNT, 1u, !v.qcfail);
     return v;
 }
-__device__ __forceinline__ Verdict pamld_decide(const DecoderParams& P, const Accumulator& accumulator, uint32_t* band_counter,
-                                                int best_index, uint32_t m, double t, double prior, double others,
-                                                double base_probability, bool uniform, uint32_t high_quality_mask, uint32_t qcfail) {
+/* the same for a mismatch mask m of the winner over at most 32 positions */
+template < bool GUARDED = false >
+__device__ __forceinline__ Verdict pamld_apply(const DecoderParams& P, const Accumulator& accumulator, uint32_t* band_counter,
+                                               int best_index, uint32_t m, double conditional_probability, double confidence,
+                                               bool uniform, uint32_t high_quality_mask, uint32_t qcfail) {
+    return pamld_apply_counted< GUARDED >(P, accumulator, band_counter, best_index, __popc(m), __popc(m & high_quality_mask), conditional_probability,
+                                          confidence, uniform, qcfail);
+}
+__device__ __forceinline__ Verdict pamld_decide_counted(const DecoderParams& P, const Accumulator& accumulator, uint32_t* band_counter,
+                                                        int best_index, int distance, int high_quality_distance, double t, double prior, double others,
+                                                        double base_probability, bool uniform, uint32_t qcfail) {
     /* when every position scores UNIFORM_BASE_QUALITY all barcodes share sigma = L x U and the
        reference's P(r|b) is the host libm constant */
     if(uniform) { base_probability = P.uniform_observation_probability; }
     const double conditional_probability = base_probability * t;
     const double p = t * prior;
     const double sigma_p = p + (others + P.adjusted_noise_probability / base_probability);
-    return pamld_apply(P, accumulator, band_counter, best_index, m, conditional_probability, p / sigma_p, uniform, high_quality_mask, qcfail);
+    return pamld_apply_counted(P, accumulator, band_counter, best_index, distance, high_quality_distance, conditional_probability, p / sigma_p, uniform, qcfail);
+}
+__device__ __forceinline__ Verdict pamld_decide(const DecoderParams& P, const Accumulator& accumulator, uint32_t* band_counter,
+                                                int best_index, uint32_t m, double t, double prior, double others,
+                                                double base_probability, bool uniform, uint32_t high_quality_mask, uint32_t qcfail) {
+    return pamld_decide_counted(P, accumulator, band_counter, best_index, __popc(m), __popc(m & high_quality_mask), t, prior, others,
+                                base_probability, uniform, qcfail);
 }
 
 /* per-position factors of an observation: what one base contributes to P0 and to a mismatch product */
@@ -814,6 +829,272 @@ pamld_kernel(const DecoderParams P, const TileArguments A) {
             const double t = subset_product< G >(table_base, m);
             const Verdict v = pamld_decide(P, S.accumulator, &S.misc[3], selection.index, m, t, e.prior, selection.rest, base_probability,
                                            uniform_positions == L, high_quality_mask, qcfail);
+            qcfail = v.qcfail;
+            A.qcfail[r] = static_cast< uint8_t >(v.qcfail);
+            store_result(A, r, v.decoded, v.distance, v.confidence, v.qcfail);
+        }
+        if(P.totals != nullptr) {
+            const unsigned live = __ballot_sync(FULL_MASK, decided);
+            const unsigned pass = __ballot_sync(FULL_MASK, decided && !qcfail);
+            if(lane == 0) {
+                atomicAdd(&S.misc[0], static_cast< uint32_t >(__popc(live)));
+                atomicAdd(&S.misc[1], static_cast< uint32_t >(__popc(pass)));
+            }
+        }
+        __syncwarp();
+    }
+    block_epilogue(S, P);
+}
+
+/* ------------------------------------------------------------------ long barcodes (33-64 nucleotides)
+   The observation and the barcodes travel in split form (LongBarcodeEntry): word 0 = positions [0, split), word 1 =
+   positions [split, L), split = 4 H with H = ceil(L / 8) groups of four positions per word. */
+constexpr int LONG_STAGE_ENTRIES = 256;          /* long barcodes per staged chunk: 8 KB */
+constexpr int LONG_MAX_WARPS = 16;
+/* the staging area of the long kernels in 16-byte units, as make_plan's blob_entries: one chunk, or two when the table streams */
+__host__ __device__ inline int long_stage_blob(int barcode_cardinality) {
+    return barcode_cardinality <= LONG_STAGE_ENTRIES ? 2 * barcode_cardinality : 4 * LONG_STAGE_ENTRIES;
+}
+
+struct LongObservation {
+    uint32_t lo[2], hi[2], nmask[2];    /* split form */
+    uint32_t qcfail;
+};
+/* the planes of read r in split form; positions past L are cleared */
+__device__ __forceinline__ LongObservation fetch_long_observation(const TileArguments& A, long long r, int split) {
+    LongObservation o;
+    uint64_t lo = 0, hi = 0, n = 0;
+    const int words = (A.nucleotides + 15) >> 4;
+    #pragma unroll
+    for(int w = 0; w < PHQ_MAX_NUCLEOTIDES / 16; ++w) {
+        if(w < words) {
+            const uint32_t b = load_stream(A.bases + w * A.pitch + r);
+            lo |= static_cast< uint64_t >(b & 0xffffu) << (16 * w);
+            hi |= static_cast< uint64_t >(b >> 16) << (16 * w);
+            n |= static_cast< uint64_t >(load_stream(A.nmask + w * A.pitch + r)) << (16 * w);
+        }
+    }
+    const uint64_t observed = A.nucleotides >= 64 ? ~0ull : ((1ull << A.nucleotides) - 1ull);
+    const uint64_t first = (1ull << split) - 1ull;
+    lo &= observed; hi &= observed; n &= observed;
+    o.lo[0] = static_cast< uint32_t >(lo & first); o.lo[1] = static_cast< uint32_t >(lo >> split);
+    o.hi[0] = static_cast< uint32_t >(hi & first); o.hi[1] = static_cast< uint32_t >(hi >> split);
+    o.nmask[0] = static_cast< uint32_t >(n & first); o.nmask[1] = static_cast< uint32_t >(n >> split);
+    o.qcfail = A.qcfail[r];
+    return o;
+}
+
+/* the long barcode table as TMA-staged chunks of 32-byte entries (BarcodeStream for LongBarcodeEntry) */
+struct LongBarcodeStream {
+    const BlockState& s;
+    const DecoderParams& P;
+    LongBarcodeEntry* stage;
+    int capacity;
+    int buffers;
+    int chunk_cardinality;
+    __device__ __forceinline__ LongBarcodeStream(const BlockState& s, const DecoderParams& P) : s(s), P(P) {
+        stage = reinterpret_cast< LongBarcodeEntry* >(s.stage);
+        capacity = P.barcode_cardinality < LONG_STAGE_ENTRIES ? P.barcode_cardinality : LONG_STAGE_ENTRIES;
+        buffers = P.barcode_cardinality <= LONG_STAGE_ENTRIES ? 1 : 2;
+        chunk_cardinality = (P.barcode_cardinality + capacity - 1) / capacity;
+    }
+    __device__ __forceinline__ int count(int chunk) const {
+        const int remaining = P.barcode_cardinality - chunk * capacity;
+        return remaining < capacity ? remaining : capacity;
+    }
+    __device__ __forceinline__ void issue(unsigned iteration) const {
+        const int chunk = iteration % chunk_cardinality;
+        const int buffer = buffers == 1 ? 0 : (iteration & 1u);
+        const uint32_t bytes = static_cast< uint32_t >(count(chunk)) * 32u;
+        mbarrier_expect_tx(&s.mbarrier[buffer], bytes);
+        tma_bulk_load(stage + static_cast< size_t >(buffer) * capacity, P.long_barcodes + static_cast< size_t >(chunk) * capacity, bytes, &s.mbarrier[buffer]);
+    }
+    __device__ __forceinline__ const LongBarcodeEntry* wait(unsigned iteration) const {
+        const int buffer = buffers == 1 ? 0 : (iteration & 1u);
+        const uint32_t use = buffers == 1 ? iteration : (iteration >> 1);
+        mbarrier_wait(&s.mbarrier[buffer], use & 1u);
+        return stage + static_cast< size_t >(buffer) * capacity;
+    }
+};
+
+/*  PAMLD scan for 33-64 nucleotides. A LANE PAIR owns one read: lane 2k + h holds the subset product tables of word h
+    of the split form (H groups, H x 4 KB per warp, as pamld_kernel< H > holds them for a whole read), so a warp keeps
+    16 reads and the shared memory a warp needs stays that of a 32-nucleotide scan. For every barcode each lane forms
+    the product over its word, the pair swaps the halves with one shuffle and both lanes hold p = (t0 * t1) * prior
+    bit for bit, so both run the same selection; the even lane queues ties and takes the decision. */
+template < int H >
+__global__ void __launch_bounds__(LONG_MAX_WARPS * WARP_SIZE, 1)
+pamld_long_kernel(const DecoderParams P, const TileArguments A) {
+    extern __shared__ __align__(256) unsigned char smem[];
+    const BlockState S = block_prologue(smem, P, true, long_stage_blob(P.barcode_cardinality));
+    const LongBarcodeStream stream(S, P);
+    const int tid = threadIdx.x;
+    const int lane = tid & 31;
+    const int warp = tid >> 5;
+    const int half = lane & 1;
+    const uint32_t window = shared_address(smem);
+    const uint32_t aligned_tables = ((window + S.plan.off_tables + 4095u) & ~4095u) - window;
+    double* const table = reinterpret_cast< double* >(smem + aligned_tables) + static_cast< size_t >(warp) * (H * 16 * WARP_SIZE) + lane;
+    const uint32_t table_base = shared_address(table);
+    const double uniform_factor = P.phred[PHRED_UNIFORM_FACTOR];
+    const int L = P.nucleotide_cardinality;
+    const int G = (L + 3) >> 2;
+    /* positions of this lane's word that the observation has */
+    const int own_positions = half == 0 ? 4 * H : L - 4 * H;
+    const uint32_t own_mask = own_positions >= 32 ? 0xffffffffu : ((1u << own_positions) - 1u);
+
+    const long long items = A.n_reads;
+    const int pairs = blockDim.x >> 1;
+    const long long tile_cardinality = (items + pairs - 1) / pairs;
+    const long long my_tiles = tile_cardinality > blockIdx.x ? (tile_cardinality - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+    const unsigned long long total_iterations = static_cast< unsigned long long >(my_tiles) * stream.chunk_cardinality;
+    unsigned iteration = 0;
+    if(tid == 0 && total_iterations > 0) { stream.issue(0); }
+    const bool resident = stream.chunk_cardinality == 1;
+    const LongBarcodeEntry* resident_stage = nullptr;
+    if(resident && total_iterations > 0) { resident_stage = stream.wait(0); }
+
+    for(long long tile = blockIdx.x; tile < tile_cardinality; tile += gridDim.x) {
+        const long long item = tile * pairs + (tid >> 1);
+        const bool valid = item < items;
+        const long long r = valid ? item : A.n_reads;
+        uint32_t o_lo = 0, o_hi = 0, nmask = 0, qcfail = 0;
+        uint32_t quality[H];
+        #pragma unroll
+        for(int g = 0; g < H; ++g) { quality[g] = 0; }
+        if(valid) {
+            const LongObservation o = fetch_long_observation(A, r, 4 * H);
+            o_lo = half ? o.lo[1] : o.lo[0]; o_hi = half ? o.hi[1] : o.hi[0]; nmask = half ? o.nmask[1] : o.nmask[0]; qcfail = o.qcfail;
+            #pragma unroll
+            for(int g = 0; g < H; ++g) {
+                const int group = half * H + g;
+                if(group < G) { quality[g] = quality_word(A, r, group); }
+            }
+        }
+
+        /* ---- this lane's factor of P0, its subset product tables and high quality positions */
+        double own_probability = 1.0;
+        uint32_t own_high_quality = 0;
+        int own_uniform = 0;
+        #pragma unroll
+        for(int g = 0; g < H; ++g) {
+            double w[4];
+            #pragma unroll
+            for(int k = 0; k < 4; ++k) {
+                const int j = g * 4 + k;
+                const uint32_t q = (quality[g] >> (8 * k)) & 0xffu;
+                if(static_cast< int >(q) >= P.high_quality_threshold) { own_high_quality |= 1u << j; }
+                const PositionFactor f = position_factor(S.phred, uniform_factor, q, (nmask >> j) & 1u);
+                own_uniform += f.uniform ? 1 : 0;
+                own_probability *= f.factor;
+                w[k] = f.ratio;
+            }
+            double* const t = table + g * 16 * WARP_SIZE;
+            const double w01 = w[0] * w[1];
+            const double w02 = w[0] * w[2];
+            const double w12 = w[1] * w[2];
+            const double w012 = w01 * w[2];
+            t[0 * WARP_SIZE] = 1.0;
+            t[1 * WARP_SIZE] = w[0];
+            t[2 * WARP_SIZE] = w[1];
+            t[3 * WARP_SIZE] = w01;
+            t[4 * WARP_SIZE] = w[2];
+            t[5 * WARP_SIZE] = w02;
+            t[6 * WARP_SIZE] = w12;
+            t[7 * WARP_SIZE] = w012;
+            t[8 * WARP_SIZE] = w[3];
+            t[9 * WARP_SIZE] = w[0] * w[3];
+            t[10 * WARP_SIZE] = w[1] * w[3];
+            t[11 * WARP_SIZE] = w01 * w[3];
+            t[12 * WARP_SIZE] = w[2] * w[3];
+            t[13 * WARP_SIZE] = w02 * w[3];
+            t[14 * WARP_SIZE] = w12 * w[3];
+            t[15 * WARP_SIZE] = w012 * w[3];
+        }
+        own_high_quality &= own_mask;
+        const double other_probability = __shfl_xor_sync(FULL_MASK, own_probability, 1);
+        const double base_probability = own_probability * other_probability;
+        const int uniform_positions = own_uniform + __shfl_xor_sync(FULL_MASK, own_uniform, 1);
+        __syncwarp();
+
+        /* ---- score every barcode (pamld_kernel's selection, on the products both lanes of the pair hold) */
+        Selection selection;
+        selection.best = 0.0; selection.rest = 0.0; selection.index = 0; selection.second = 0;
+        uint32_t near_blocks = 0u;
+        for(int chunk = 0; chunk < stream.chunk_cardinality; ++chunk) {
+            const LongBarcodeEntry* stage;
+            if(resident) {
+                stage = resident_stage;
+            } else {
+                if(tid == 0 && iteration + 1 < total_iterations) { stream.issue(iteration + 1); }
+                stage = stream.wait(iteration);
+            }
+            const int count = stream.count(chunk);
+            const int first = chunk * stream.capacity;
+            int i = 0;
+            #pragma unroll 2
+            for(; i + 4 <= count; i += 4) {
+                double p[4];
+                #pragma unroll
+                for(int u = 0; u < 4; ++u) {
+                    const uint2 planes = reinterpret_cast< const uint2* >(stage + i + u)[half];
+                    const double own = subset_product< H >(table_base, mismatch_mask(o_lo, o_hi, nmask, planes.x, planes.y));
+                    const double other = __shfl_xor_sync(FULL_MASK, own, 1);
+                    p[u] = (own * other) * stage[i + u].prior;       /* a product does not depend on the order of its factors */
+                }
+                note_block(near_blocks, __double2hiint(selection.best), top_high(p[0], p[1], p[2], p[3]), first + i, P.tie_block_shift);
+                select_four(selection, p[0], p[1], p[2], p[3], first + i);
+            }
+            for(; i < count; ++i) {
+                const uint2 planes = reinterpret_cast< const uint2* >(stage + i)[half];
+                const double own = subset_product< H >(table_base, mismatch_mask(o_lo, o_hi, nmask, planes.x, planes.y));
+                const double other = __shfl_xor_sync(FULL_MASK, own, 1);
+                const double p = (own * other) * stage[i].prior;
+                note_block(near_blocks, __double2hiint(selection.best), __double2hiint(p), first + i, P.tie_block_shift);
+                select_one(selection, p, first + i);
+            }
+            if(!resident) {
+                __syncthreads();
+                ++iteration;
+            }
+        }
+
+        /* ---- ties go to pamld_long_tie_kernel, which reads the observation from the tile again: the record keeps the
+           scan's sums, P0 and the flagged runs of barcodes */
+        const bool tied = valid && (selection.second + 1 >= __double2hiint(selection.best));
+        const bool queued = tied && half == 0;
+        const unsigned queue = __ballot_sync(FULL_MASK, queued);
+        if(queue) {
+            unsigned slot = 0;
+            if(lane == 0) { slot = atomicAdd(P.tie_count, static_cast< unsigned >(__popc(queue))); }
+            slot = __shfl_sync(FULL_MASK, slot, 0);
+            if(queued) {
+                TieRecord record;
+                memset(&record, 0, sizeof(record));
+                record.best = selection.best;
+                record.rest = selection.rest;
+                record.base_probability = base_probability;
+                record.uniform = uniform_positions == L ? 1u : 0u;
+                record.read = static_cast< uint32_t >(r);
+                record.candidate_count = TIE_BLOCKS;
+                record.candidate[0] = near_blocks;
+                record.candidate[1] = static_cast< uint32_t >(P.tie_block_shift);
+                P.tie_record[slot + __popc(queue & ((1u << lane) - 1u))] = record;
+            }
+        }
+
+        /* ---- the decision: both lanes form their half of the winner's product and mismatch counts */
+        const LongBarcodeEntry& winner = P.long_barcodes[selection.index];
+        const uint2 planes = reinterpret_cast< const uint2* >(&winner)[half];
+        const uint32_t m = mismatch_mask(o_lo, o_hi, nmask, planes.x, planes.y);
+        const double own_t = subset_product< H >(table_base, m);
+        const double other_t = __shfl_xor_sync(FULL_MASK, own_t, 1);
+        const int distance = __popc(m) + __shfl_xor_sync(FULL_MASK, __popc(m), 1);
+        const int high_quality_distance = __popc(m & own_high_quality) + __shfl_xor_sync(FULL_MASK, __popc(m & own_high_quality), 1);
+        const bool decided = valid && !tied && half == 0;
+        if(decided) {
+            const Verdict v = pamld_decide_counted(P, S.accumulator, &S.misc[3], selection.index, distance, high_quality_distance, own_t * other_t, winner.prior,
+                                                   selection.rest, base_probability, uniform_positions == L, qcfail);
             qcfail = v.qcfail;
             A.qcfail[r] = static_cast< uint8_t >(v.qcfail);
             store_result(A, r, v.decoded, v.distance, v.confidence, v.qcfail);
@@ -2646,6 +2927,216 @@ pamld_tie_kernel(const DecoderParams P, const TileArguments A) {
     if(tid == 2 && P.diagnostics != nullptr && blockIdx.x == 0 && tie_cardinality) { atomicAdd(&P.diagnostics[DIAG_EXACT_PATH], static_cast< unsigned long long >(tie_cardinality)); }
 }
 
+/*  The tie pass of pamld_long_kernel: pamld_tie_kernel's thread per queued read, with the observation read again from
+    the tile through the record's read index (a record has no room for 64 quality bytes) and the candidates taken from
+    the flagged runs of barcodes, the only form that scan queues. Position j of the split form is bit j of word 0 for
+    j < 4 H and bit j - 4 H of word 1 after it; the Kahan sums run over positions 0 .. L - 1 in order. */
+__host__ __device__ constexpr size_t long_tie_shared_bytes(int N) {
+    return 4096 + TIE_SCORE_ENTRIES * 8 + 128 * 8
+         + (N <= TIE_STAGE_ENTRIES ? static_cast< size_t >(N) * sizeof(LongBarcodeEntry) : 0)
+         + static_cast< size_t >(tie_accumulator_rows(N)) * (ACC_F64_COLUMNS * 8 + ACC_U64_COLUMNS * 4);
+}
+/* bit j of the split form of m moved to bit 10 (the mismatch bit of a score address); j is a constant after unrolling */
+template < int H >
+__device__ __forceinline__ uint32_t long_moved(uint32_t m0, uint32_t m1, int j) {
+    const int at = j < 4 * H ? j : j - 4 * H;
+    const uint32_t word = j < 4 * H ? m0 : m1;
+    return at <= 10 ? (word << (at <= 10 ? 10 - at : 0)) : (word >> (at <= 10 ? 0 : at - 10));
+}
+/* sigma_q of two candidates (tie_sigma_pair over the split form) */
+template < int H >
+__device__ __forceinline__ void long_tie_sigma_pair(const uint32_t (&score_address)[8 * H], uint32_t a0, uint32_t a1, uint32_t b0, uint32_t b1, int L,
+                                                    double& sigma0, double& sigma1) {
+    double s0 = 0.0, c0 = 0.0, s1 = 0.0, c1 = 0.0;
+    #pragma unroll
+    for(int j = 0; j < 8 * H; ++j) {
+        if(j >= 8 * (H - 1) && j >= L) { break; }
+        uint32_t address0, address1;
+        asm("lop3.b32 %0, %1, 0x400, %2, 0xEA;" : "=r"(address0) : "r"(long_moved< H >(a0, a1, j)), "r"(score_address[j]));
+        asm("lop3.b32 %0, %1, 0x400, %2, 0xEA;" : "=r"(address1) : "r"(long_moved< H >(b0, b1, j)), "r"(score_address[j]));
+        double value0, value1;
+        asm("ld.shared.f64 %0, [%1];" : "=d"(value0) : "r"(address0));
+        asm("ld.shared.f64 %0, [%1];" : "=d"(value1) : "r"(address1));
+        const double y0 = __dsub_rn(value0, c0);
+        const double y1 = __dsub_rn(value1, c1);
+        const double t0 = __dadd_rn(s0, y0);
+        const double t1 = __dadd_rn(s1, y1);
+        c0 = __dsub_rn(__dsub_rn(t0, s0), y0);
+        c1 = __dsub_rn(__dsub_rn(t1, s1), y1);
+        s0 = t0;
+        s1 = t1;
+    }
+    sigma0 = s0;
+    sigma1 = s1;
+}
+/* the mismatch product over the counted positions (tie_product over the split form) */
+template < int H >
+__device__ __forceinline__ double long_tie_product(const uint32_t (&score_address)[8 * H], uint32_t ratio_table, uint32_t counted0, uint32_t counted1, int L) {
+    double t = 1.0;
+    #pragma unroll
+    for(int j = 0; j < 8 * H; ++j) {
+        if(j >= 8 * (H - 1) && j >= L) { break; }
+        if(((j < 4 * H ? counted0 : counted1) >> (j < 4 * H ? j : j - 4 * H)) & 1u) {
+            double value;
+            asm("ld.shared.f64 %0, [%1];" : "=d"(value) : "r"(ratio_table + (score_address[j] & 0x3f8u)));
+            t *= value;
+        }
+    }
+    return t;
+}
+
+template < int H >
+__global__ void __launch_bounds__(TIE_THREADS, 2)
+pamld_long_tie_kernel(const DecoderParams P, const TileArguments A) {
+    extern __shared__ __align__(16) unsigned char tie_smem[];
+    __shared__ uint32_t block_counter[4];
+    const int tid = threadIdx.x;
+    const int lane = tid & 31;
+    const int N = P.barcode_cardinality;
+    const unsigned tie_cardinality = *P.tie_count;
+    if(blockIdx.x * TIE_THREADS >= tie_cardinality) { return; }
+
+    /* ---- shared memory: score table (4 KB aligned), mismatch ratios, the barcode table when it is small, accumulator rows */
+    const uint32_t window = shared_address(tie_smem);
+    const uint32_t slack = (4096u - (window & 4095u)) & 4095u;
+    double* const score = reinterpret_cast< double* >(tie_smem + slack);
+    double* const ratio = score + TIE_SCORE_ENTRIES;
+    unsigned char* cursor = reinterpret_cast< unsigned char* >(ratio + 128);
+    const uint32_t score_table = window + slack;
+    const uint32_t ratio_table = score_table + TIE_SCORE_ENTRIES * 8;
+    const double uniform_quality = P.phred[PHRED_UNIFORM_QUALITY];
+    const double base = P.phred[PHRED_BASE];
+    for(int i = tid; i < TIE_SCORE_ENTRIES; i += blockDim.x) {
+        const int q = i & 127;
+        score[i] = q == 0 ? 0.0 : ((i >> 8) ? uniform_quality : (((i >> 7) & 1) ? static_cast< double >(q) : P.phred[PHRED_TRUE_POSITIVE_QUALITY + q]));
+    }
+    for(int i = tid; i < 128; i += blockDim.x) { ratio[i] = P.phred[PHRED_MISMATCH_RATIO + i]; }
+    const LongBarcodeEntry* barcodes = P.long_barcodes;
+    if(N <= TIE_STAGE_ENTRIES) {
+        uint4* const stage = reinterpret_cast< uint4* >(cursor);
+        for(int i = tid; i < 2 * N; i += blockDim.x) { stage[i] = reinterpret_cast< const uint4* >(P.long_barcodes)[i]; }
+        barcodes = reinterpret_cast< const LongBarcodeEntry* >(cursor);
+        cursor += static_cast< size_t >(N) * sizeof(LongBarcodeEntry);
+    }
+    if(tid < 4) { block_counter[tid] = 0; }
+    const int accumulator_rows = tie_accumulator_rows(N);
+    Accumulator accumulator;
+    accumulator.shared_u32 = nullptr;
+    accumulator.shared_f64 = nullptr;
+    accumulator.global_u64 = P.acc_u64;
+    accumulator.global_f64 = P.acc_f64;
+    if(accumulator_rows > 0) {
+        accumulator.shared_f64 = reinterpret_cast< double* >(cursor);
+        accumulator.shared_u32 = reinterpret_cast< uint32_t* >(accumulator.shared_f64 + accumulator_rows * ACC_F64_COLUMNS);
+        for(int i = tid; i < accumulator_rows * ACC_F64_COLUMNS; i += blockDim.x) { accumulator.shared_f64[i] = 0.0; }
+        for(int i = tid; i < accumulator_rows * ACC_U64_COLUMNS; i += blockDim.x) { accumulator.shared_u32[i] = 0u; }
+    }
+    __syncthreads();
+
+    const int L = P.nucleotide_cardinality;
+    const int G = (L + 3) >> 2;
+    for(;;) {
+        unsigned first_item = 0;
+        if(lane == 0) { first_item = atomicAdd(P.tie_count + 1, 32u); }
+        first_item = __shfl_sync(FULL_MASK, first_item, 0);
+        if(first_item >= tie_cardinality) { break; }
+        const unsigned item = first_item + lane;
+        const bool live = item < tie_cardinality;
+        const TieRecord& record = P.tie_record[live ? item : 0u];
+        const long long r = live ? static_cast< long long >(record.read) : 0;
+        LongObservation o;
+        uint32_t score_address[8 * H];
+        uint32_t high_quality[2] = { 0u, 0u };
+        o.lo[0] = o.lo[1] = o.hi[0] = o.hi[1] = o.nmask[0] = o.nmask[1] = 0u;
+        #pragma unroll
+        for(int j = 0; j < 8 * H; ++j) { score_address[j] = score_table; }
+        if(live) {
+            o = fetch_long_observation(A, r, 4 * H);
+            #pragma unroll
+            for(int g = 0; g < 2 * H; ++g) {
+                const uint32_t word = g < G ? quality_word(A, r, g) : 0u;
+                #pragma unroll
+                for(int k = 0; k < 4; ++k) {
+                    const int j = 4 * g + k;
+                    const int half = j < 4 * H ? 0 : 1;
+                    const int at = j - 4 * H * half;
+                    const uint32_t raw = (word >> (8 * k)) & 0xffu;
+                    if(j < L && static_cast< int >(raw) >= P.high_quality_threshold) { high_quality[half] |= 1u << at; }
+                    score_address[j] = score_table + phred_quality(raw) * 8u + ((o.nmask[half] >> at) & 1u) * 2048u;
+                }
+            }
+        }
+
+        /* ---- the candidates: the members of the flagged runs */
+        const uint32_t run = 4u << (record.candidate[1] & 31u);
+        uint32_t pending_runs = live ? record.candidate[0] : 0u;
+        uint32_t next = 0u, last = 0u;
+        Candidate best;
+        best.prior = 0; best.sigma = 0; best.index = -1;
+        auto pull = [&]() -> int {
+            for(;;) {
+                if(next >= last) {
+                    if(pending_runs == 0u) { return -1; }
+                    const uint32_t bit = static_cast< uint32_t >(__ffs(static_cast< int >(pending_runs)) - 1);
+                    pending_runs &= pending_runs - 1u;
+                    next = bit * run;
+                    last = min(next + run, static_cast< uint32_t >(N));
+                    continue;
+                }
+                return static_cast< int >(next++);
+            }
+        };
+        for(;;) {
+            const int b0 = pull();
+            if(b0 < 0) { break; }
+            const int b1 = pull();
+            const LongBarcodeEntry e0 = barcodes[b0];
+            const LongBarcodeEntry e1 = barcodes[max(b1, 0)];
+            const uint32_t m00 = ((o.lo[0] ^ e0.lo0) | (o.hi[0] ^ e0.hi0)) | o.nmask[0];
+            const uint32_t m01 = ((o.lo[1] ^ e0.lo1) | (o.hi[1] ^ e0.hi1)) | o.nmask[1];
+            const uint32_t m10 = ((o.lo[0] ^ e1.lo0) | (o.hi[0] ^ e1.hi0)) | o.nmask[0];
+            const uint32_t m11 = ((o.lo[1] ^ e1.lo1) | (o.hi[1] ^ e1.hi1)) | o.nmask[1];
+            Candidate first, second;
+            long_tie_sigma_pair< H >(score_address, m00, m01, m10, m11, L, first.sigma, second.sigma);
+            first.prior = e0.prior;
+            first.index = b0;
+            second.prior = e1.prior;
+            second.index = b1;                              /* -1 = none: beats() lets it lose */
+            if(beats(second, first, base)) { first = second; }
+            if(beats(first, best, base)) { best = first; }
+        }
+
+        /* ---- the decision (pamld.cpp:87-122) */
+        bool passes = false;
+        if(live) {
+            const int winner = max(best.index, 0);
+            const LongBarcodeEntry e = barcodes[winner];
+            const uint32_t m0 = ((o.lo[0] ^ e.lo0) | (o.hi[0] ^ e.hi0)) | o.nmask[0];
+            const uint32_t m1 = ((o.lo[1] ^ e.lo1) | (o.hi[1] ^ e.hi1)) | o.nmask[1];
+            const double t = long_tie_product< H >(score_address, ratio_table, m0 & ~o.nmask[0], m1 & ~o.nmask[1], L);
+            /* everything but the winner: the scan's total minus the winner (see pamld_tie_kernel) */
+            const double others = (record.best - t * e.prior) + record.rest;
+            const Verdict v = pamld_decide_counted(P, accumulator, &block_counter[3], winner, __popc(m0) + __popc(m1),
+                                                   __popc(m0 & high_quality[0]) + __popc(m1 & high_quality[1]), t, e.prior, others,
+                                                   record.base_probability, record.uniform != 0u, o.qcfail);
+            A.qcfail[r] = static_cast< uint8_t >(v.qcfail);
+            store_result(A, r, v.decoded, v.distance, v.confidence, v.qcfail);
+            passes = !v.qcfail;
+        }
+        const unsigned decided = __ballot_sync(FULL_MASK, live);
+        const unsigned passing = __ballot_sync(FULL_MASK, passes);
+        if(lane == 0) {
+            atomicAdd(&block_counter[0], static_cast< uint32_t >(__popc(decided)));
+            if(passing) { atomicAdd(&block_counter[1], static_cast< uint32_t >(__popc(passing))); }
+        }
+    }
+    __syncthreads();
+    if(tid < 2 && P.totals != nullptr && block_counter[tid]) { atomicAdd(&P.totals[tid], static_cast< unsigned long long >(block_counter[tid])); }
+    if(accumulator_rows > 0) { flush_accumulators(accumulator, accumulator_rows, P); }
+    if(tid == 3 && P.diagnostics != nullptr && block_counter[3]) { atomicAdd(&P.diagnostics[DIAG_THRESHOLD_BAND], static_cast< unsigned long long >(block_counter[3])); }
+    if(tid == 2 && P.diagnostics != nullptr && blockIdx.x == 0 && tie_cardinality) { atomicAdd(&P.diagnostics[DIAG_EXACT_PATH], static_cast< unsigned long long >(tie_cardinality)); }
+}
+
 /* ------------------------------------------------------------------ MDD */
 template < int SEGMENTS >      /* 0 = run-time segment count */
 __global__ void __launch_bounds__(MAX_WARPS * WARP_SIZE, 2)
@@ -2736,6 +3227,119 @@ mdd_kernel(const DecoderParams P, const TileArguments A) {
             }
         }
 
+        if(valid) {
+            int decoded = 0, distance = 0;
+            if(exact_index >= 0) { decoded = exact_index + 1; }
+            else if(found_index >= 0) { decoded = found_index + 1; distance = found_distance; }
+            if(decoded == 0) { qcfail = 1; }
+            if(decoded > 0 && distance > 0) {
+                S.accumulator.add_pair(decoded, ACC_DISTANCE, ACC_PF_DISTANCE, static_cast< uint32_t >(distance), !qcfail);
+            }
+            S.accumulator.add_pair(decoded, ACC_COUNT, ACC_PF_COUNT, 1u, !qcfail);
+            A.qcfail[r] = static_cast< uint8_t >(qcfail);
+            store_result(A, r, decoded, distance, 0.0, qcfail);
+        }
+        if(P.totals != nullptr) {
+            const unsigned live = __ballot_sync(FULL_MASK, valid);
+            const unsigned pass = __ballot_sync(FULL_MASK, valid && !qcfail);
+            if(lane == 0) {
+                atomicAdd(&S.misc[0], static_cast< uint32_t >(__popc(live)));
+                atomicAdd(&S.misc[1], static_cast< uint32_t >(__popc(pass)));
+            }
+        }
+    }
+    block_epilogue(S, P);
+}
+
+/* mdd_kernel for 33-64 nucleotides: the same scan over the split form (LongBarcodeEntry, segment_mask / segment_mask_long) */
+template < int SEGMENTS >      /* 0 = run-time segment count */
+__global__ void __launch_bounds__(MAX_WARPS * WARP_SIZE, 2)
+mdd_long_kernel(const DecoderParams P, const TileArguments A) {
+    extern __shared__ __align__(256) unsigned char smem[];
+    const BlockState S = block_prologue(smem, P, false, long_stage_blob(P.barcode_cardinality));
+    const LongBarcodeStream stream(S, P);
+    const int tid = threadIdx.x;
+    const int lane = tid & 31;
+    const int L = P.nucleotide_cardinality;
+    const int split = P.long_split;
+    const int segment_cardinality = SEGMENTS > 0 ? SEGMENTS : P.segment_cardinality;
+    const uint32_t all_positions[2] = { split >= 32 ? 0xffffffffu : ((1u << split) - 1u), L - split >= 32 ? 0xffffffffu : ((1u << (L - split)) - 1u) };
+
+    const long long item_cardinality = A.n_reads;
+    const long long tile_cardinality = (item_cardinality + blockDim.x - 1) / blockDim.x;
+    const long long my_tiles = tile_cardinality > blockIdx.x ? (tile_cardinality - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+    const unsigned long long total_iterations = static_cast< unsigned long long >(my_tiles) * stream.chunk_cardinality;
+    unsigned iteration = 0;
+    if(tid == 0 && total_iterations > 0) { stream.issue(0); }
+    const bool resident = stream.chunk_cardinality == 1;
+    const LongBarcodeEntry* resident_stage = nullptr;
+    if(resident && total_iterations > 0) { resident_stage = stream.wait(0); }
+
+    for(long long tile = blockIdx.x; tile < tile_cardinality; tile += gridDim.x) {
+        const long long r = tile * blockDim.x + tid;
+        const bool valid = r < item_cardinality;
+        LongObservation o;
+        o.lo[0] = o.lo[1] = o.hi[0] = o.hi[1] = o.nmask[0] = o.nmask[1] = 0u;
+        o.qcfail = 0;
+        uint32_t present[2] = { 0u, 0u }, masked[2] = { 0u, 0u };
+        if(valid) {
+            o = fetch_long_observation(A, r, split);
+            /* absent positions: ambiguous with both base bits set (mdd_kernel) */
+            #pragma unroll
+            for(int h = 0; h < 2; ++h) { present[h] = ~(o.nmask[h] & o.lo[h] & o.hi[h]) & all_positions[h]; }
+            if(P.quality_masking_threshold > 0) {
+                for(int g = 0; g < P.quality_word_cardinality; ++g) {
+                    const uint32_t qw = quality_word(A, r, g);
+                    #pragma unroll
+                    for(int k = 0; k < 4; ++k) {
+                        const int j = g * 4 + k;
+                        if(static_cast< int >((qw >> (8 * k)) & 0xffu) < P.quality_masking_threshold) {
+                            if(j < split) { masked[0] |= 1u << j; } else { masked[1] |= 1u << (j - split); }
+                        }
+                    }
+                }
+                masked[0] &= present[0];
+                masked[1] &= present[1];
+            }
+        }
+        const bool complete = present[0] == all_positions[0] && present[1] == all_positions[1];
+        const uint32_t qcfail_in = o.qcfail;
+
+        int exact_index = -1, found_index = -1, found_distance = 0;
+        for(int chunk = 0; chunk < stream.chunk_cardinality; ++chunk) {
+            const LongBarcodeEntry* stage;
+            if(resident) {
+                stage = resident_stage;
+            } else {
+                if(tid == 0 && iteration + 1 < total_iterations) { stream.issue(iteration + 1); }
+                stage = stream.wait(iteration);
+            }
+            const int count = stream.count(chunk);
+            const int first = chunk * stream.capacity;
+            #pragma unroll 4
+            for(int i = 0; i < count; ++i) {
+                const uint4 raw = *reinterpret_cast< const uint4* >(stage + i);
+                const uint32_t m0 = ((o.lo[0] ^ raw.x) | (o.hi[0] ^ raw.y)) | o.nmask[0];
+                const uint32_t m1 = ((o.lo[1] ^ raw.z) | (o.hi[1] ^ raw.w)) | o.nmask[1];
+                const uint32_t error0 = (m0 | masked[0]) & present[0];
+                const uint32_t error1 = (m1 | masked[1]) & present[1];
+                bool within = true;
+                #pragma unroll
+                for(int s = 0; s < (SEGMENTS > 0 ? SEGMENTS : PHQ_MAX_SEGMENTS); ++s) {
+                    if(s < segment_cardinality) {
+                        within = within && (__popc(error0 & P.segment_mask[s]) + __popc(error1 & P.segment_mask_long[s]) <= P.distance_tolerance[s]);
+                    }
+                }
+                if(complete && (m0 | m1) == 0u && exact_index < 0) { exact_index = first + i; }
+                if(within && found_index < 0) { found_index = first + i; found_distance = __popc(error0) + __popc(error1); }
+            }
+            if(!resident) {
+                __syncthreads();
+                ++iteration;
+            }
+        }
+
+        uint32_t qcfail = qcfail_in;
         if(valid) {
             int decoded = 0, distance = 0;
             if(exact_index >= 0) { decoded = exact_index + 1; }
@@ -3100,6 +3704,44 @@ cudaError_t launch_pamld_fast_grid(const DecoderParams& params, const TileArgume
     return cudaErrorInvalidValue;
 }
 
+/* the long scan (H = ceil(L / 8) groups per lane), then its tie pass */
+template < int H >
+cudaError_t launch_pamld_long(const DecoderParams& params, const TileArguments& tile, const LaunchGeometry& geometry, cudaStream_t stream) {
+    const SharedPlan plan = make_plan(params.barcode_cardinality, true, long_stage_blob(params.barcode_cardinality));
+    const size_t per_warp = static_cast< size_t >(H) * 16 * WARP_SIZE * sizeof(double);
+    if(plan.fixed_bytes + per_warp > geometry.shared_memory_per_block_optin) { return cudaErrorInvalidConfiguration; }
+    int warps = static_cast< int >((geometry.shared_memory_per_block_optin - plan.fixed_bytes) / per_warp);
+    warps = warps > LONG_MAX_WARPS ? LONG_MAX_WARPS : warps;
+    const size_t bytes = plan.fixed_bytes + per_warp * warps;
+    cudaError_t status = cudaFuncSetAttribute(pamld_long_kernel< H >, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast< int >(bytes));
+    if(status != cudaSuccess) { return status; }
+    const int reads_per_tile = warps * WARP_SIZE / 2;
+    const long long tiles = (tile.n_reads + reads_per_tile - 1) / reads_per_tile;
+    const int grid = static_cast< int >(tiles < geometry.multiprocessor_count ? tiles : geometry.multiprocessor_count);
+    status = cudaMemsetAsync(params.tie_count, 0, 2 * sizeof(unsigned), stream);      /* the tie queue's length and the tie pass' work counter */
+    if(status != cudaSuccess) { return status; }
+    pamld_long_kernel< H ><<< grid, warps * WARP_SIZE, bytes, stream >>>(params, tile);
+    status = cudaGetLastError();
+    if(status != cudaSuccess) { return status; }
+    const size_t tie_bytes = long_tie_shared_bytes(params.barcode_cardinality);
+    status = cudaFuncSetAttribute(pamld_long_tie_kernel< H >, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast< int >(tie_bytes));
+    if(status != cudaSuccess) { return status; }
+    pamld_long_tie_kernel< H ><<< geometry.multiprocessor_count * 2, TIE_THREADS, tie_bytes, stream >>>(params, tile);
+    return cudaGetLastError();
+}
+
+template < int SEGMENTS >
+cudaError_t launch_mdd_long_as(const DecoderParams& params, const TileArguments& tile, const LaunchGeometry& geometry, cudaStream_t stream) {
+    const size_t bytes = make_plan(params.barcode_cardinality, false, long_stage_blob(params.barcode_cardinality)).fixed_bytes;
+    const int threads = 256;
+    const long long tiles = (tile.n_reads + threads - 1) / threads;
+    const long long resident = static_cast< long long >(geometry.multiprocessor_count) * 4;
+    const cudaError_t status = cudaFuncSetAttribute(mdd_long_kernel< SEGMENTS >, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast< int >(bytes));
+    if(status != cudaSuccess) { return status; }
+    mdd_long_kernel< SEGMENTS ><<< static_cast< int >(tiles < resident ? tiles : resident), threads, bytes, stream >>>(params, tile);
+    return cudaGetLastError();
+}
+
 }   /* namespace */
 
 static cudaError_t launch_pamld_whitelist(const DecoderParams& params, const TileArguments& tile, const LaunchGeometry& geometry, cudaStream_t stream) {
@@ -3124,6 +3766,15 @@ static cudaError_t launch_pamld_whitelist(const DecoderParams& params, const Til
 
 cudaError_t launch_pamld(const DecoderParams& params, const TileArguments& tile, const LaunchGeometry& geometry, cudaStream_t stream) {
     if(tile.n_reads <= 0) { return cudaSuccess; }
+    if(params.nucleotide_cardinality > LONG_NUCLEOTIDES) {
+        switch((params.nucleotide_cardinality + 7) / 8) {
+            case 5: return launch_pamld_long< 5 >(params, tile, geometry, stream);
+            case 6: return launch_pamld_long< 6 >(params, tile, geometry, stream);
+            case 7: return launch_pamld_long< 7 >(params, tile, geometry, stream);
+            case 8: return launch_pamld_long< 8 >(params, tile, geometry, stream);
+            default: return cudaErrorInvalidValue;
+        }
+    }
     if(params.whitelist != nullptr) { return launch_pamld_whitelist(params, tile, geometry, stream); }
     if(params.fast_barcodes != nullptr) {
         /* f32 prefilter scan first (see pamld_fast_kernel); the api only offers it for the shapes handled here */
@@ -3195,6 +3846,13 @@ static cudaError_t launch_mdd_scan(const DecoderParams& params, const TileArgume
 
 cudaError_t launch_mdd(const DecoderParams& params, const TileArguments& tile, const LaunchGeometry& geometry, cudaStream_t stream) {
     if(tile.n_reads <= 0) { return cudaSuccess; }
+    if(params.nucleotide_cardinality > LONG_NUCLEOTIDES) {
+        switch(params.segment_cardinality) {
+            case 1: return launch_mdd_long_as< 1 >(params, tile, geometry, stream);
+            case 2: return launch_mdd_long_as< 2 >(params, tile, geometry, stream);
+            default: return launch_mdd_long_as< 0 >(params, tile, geometry, stream);
+        }
+    }
     if(params.mdd_tables == nullptr) { return launch_mdd_scan(params, tile, geometry, stream); }
     /* lookup kernel, then the scan kernel over the reads it queued (short tokens) */
     int* const queue = reinterpret_cast< int* >(reinterpret_cast< unsigned char* >(params.tie_record));
@@ -3254,7 +3912,10 @@ cudaError_t launch_count(const DecoderParams& params, const TileArguments& tile,
 void describe_kernels(const DecoderParams& params, int algorithm, char* buffer, size_t capacity) {
     if(buffer == nullptr || capacity == 0) { return; }
     const int L = params.nucleotide_cardinality;
-    if(algorithm == 0) {
+    if(algorithm <= 1 && L > LONG_NUCLEOTIDES) {
+        if(algorithm == 0) { snprintf(buffer, capacity, "pamld_long_kernel<%d> + pamld_long_tie_kernel<%d>", (L + 7) / 8, (L + 7) / 8); }
+        else { snprintf(buffer, capacity, "mdd_long_kernel<%d>", params.segment_cardinality <= 2 ? params.segment_cardinality : 0); }
+    } else if(algorithm == 0) {
         const bool grid = params.grid != nullptr && grid_shape_supported(params.grid_split, L);
         if(params.whitelist != nullptr) {
             snprintf(buffer, capacity, "pamld_whitelist_kernel + pamld_tie_kernel<4>");

@@ -32,6 +32,21 @@ struct __align__(16) FastEntry {
     uint32_t pad;
 };
 
+/*  Decoders of more than LONG_NUCLEOTIDES positions (up to PHQ_MAX_NUCLEOTIDES) take the long kernels
+    (pamld_long_kernel, pamld_long_tie_kernel, mdd_long_kernel) and this table instead of the 16-byte one. Their
+    positions travel in SPLIT FORM, two 32-bit words per plane: word 0 holds positions [0, split), word 1 positions
+    [split, L), split = long_split(L) = 4 x ceil(L / 8), so each word covers at most ceil(L / 8) groups of four
+    positions and the PAMLD scan gives one word to each lane of a lane pair. */
+constexpr int LONG_NUCLEOTIDES = 32;
+__host__ __device__ inline int long_split(int nucleotides) { return 4 * ((nucleotides + 7) / 8); }
+struct __align__(16) LongBarcodeEntry {
+    uint32_t lo0, hi0;      /* low / high bit-plane of positions [0, split) */
+    uint32_t lo1, hi1;      /* of positions [split, L), position split + j = bit j */
+    double prior;
+    double pad;
+};
+static_assert(sizeof(LongBarcodeEntry) == 32, "one long barcode entry is 32 bytes");
+
 /* offsets into the f64 Phred table uploaded once per handle */
 enum {
     PHRED_MATCH_FACTOR   = 0,       /* [128]  B ^ true_positive_quality[q]      (q = 0 -> 1)            */
@@ -154,6 +169,10 @@ struct DecoderParams {
     int32_t tie_block_shift;                    /* log2 of the blocks of four barcodes (grid entries) one bit of a TIE_BLOCKS mask stands for */
     uint32_t* tie_pool;                         /* candidates of the reads that name more than a record holds; cursor = tie_count[3] */
     uint32_t tie_pool_capacity;
+    /* decoders of more than LONG_NUCLEOTIDES positions: `barcodes` is NULL, segment_mask holds word 0 of the split form */
+    const LongBarcodeEntry* long_barcodes;      /* [N] device */
+    int32_t long_split;                         /* long_split(nucleotide_cardinality) */
+    uint32_t segment_mask_long[PHQ_MAX_SEGMENTS];   /* word 1 of each segment's mask in split form (MDD) */
 };
 
 struct TileArguments {

@@ -1,6 +1,8 @@
 /*  pack.cu — the feed -> tile kernel (pack.cuh). Lane = read. */
 #include "pack.cuh"
 
+#include <type_traits>
+
 namespace phq {
 namespace {
 
@@ -94,9 +96,13 @@ __device__ __forceinline__ Base fetch(const TokenView& plan, const uint8_t* tabl
     return b;
 }
 
+/*  MAX = the most nucleotides the instantiation packs: 32 (one 32-bit word per plane) or PHQ_MAX_NUCLEOTIDES (64-bit
+    planes, for decoders of more than 32 nucleotides) */
+template < int MAX >
 __global__ void __launch_bounds__(256)
 pack_kernel(const __grid_constant__ PackPlan pack_plan, const long long n_reads, uint32_t* __restrict__ bases, uint16_t* __restrict__ nmask,
             uint32_t* __restrict__ quality, const long long pitch) {
+    typedef typename std::conditional< (MAX <= 32), uint32_t, uint64_t >::type Plane;
     __shared__ uint8_t table[96];
     if(threadIdx.x < 80) { table[threadIdx.x] = ASCII_TO_BAM[threadIdx.x]; }
     else if(threadIdx.x < 96) { table[threadIdx.x] = BAM_COMPLEMENT[threadIdx.x - 80]; }
@@ -104,21 +110,22 @@ pack_kernel(const __grid_constant__ PackPlan pack_plan, const long long n_reads,
     const TokenView plan = view_of(pack_plan);
     const int L = pack_plan.nucleotide_cardinality;
     for(long long r = blockIdx.x * static_cast< long long >(blockDim.x) + threadIdx.x; r < n_reads; r += static_cast< long long >(gridDim.x) * blockDim.x) {
-        uint32_t lo = 0, hi = 0, ambiguous = 0;
-        uint32_t phred[PHQ_MAX_NUCLEOTIDES / 4];
+        Plane lo = 0, hi = 0, ambiguous = 0;
+        uint32_t phred[MAX / 4];
         #pragma unroll
-        for(int w = 0; w < PHQ_MAX_NUCLEOTIDES / 4; ++w) { phred[w] = 0; }
+        for(int w = 0; w < MAX / 4; ++w) { phred[w] = 0; }
         for(int s = 0; s < pack_plan.segment_cardinality; ++s) {
             const int expected = pack_plan.segment_offset[s + 1] - pack_plan.segment_offset[s];
             const int length = observed_length(plan, table, r, s);
             for(int i = 0; i < expected; ++i) {
                 const int j = pack_plan.segment_offset[s] + i;
+                const Plane bit = static_cast< Plane >(1) << j;
                 Base b;
                 if(i < length) {
                     b = fetch(plan, table, r, s, i);
                 } else if(!pack_plan.stale_semantics) {
                     /* absent position (phq_pack): quality PHQ_ABSENT_QUALITY, ambiguous with both base bits set */
-                    lo |= 1u << j; hi |= 1u << j; ambiguous |= 1u << j;
+                    lo |= bit; hi |= bit; ambiguous |= bit;
                     phred[j >> 2] |= static_cast< uint32_t >(PHQ_ABSENT_QUALITY) << (8 * (j & 3));
                     continue;
                 } else if(i == length) {
@@ -134,22 +141,32 @@ pack_kernel(const __grid_constant__ PackPlan pack_plan, const long long n_reads,
                 }
                 switch(b.code) {
                     case 1: break;
-                    case 2: lo |= 1u << j; break;
-                    case 4: hi |= 1u << j; break;
-                    case 8: lo |= 1u << j; hi |= 1u << j; break;
-                    default: ambiguous |= 1u << j; break;
+                    case 2: lo |= bit; break;
+                    case 4: hi |= bit; break;
+                    case 8: lo |= bit; hi |= bit; break;
+                    default: ambiguous |= bit; break;
                 }
                 phred[j >> 2] |= b.quality << (8 * (j & 3));
             }
         }
-        bases[r] = (lo & 0xffffu) | ((hi & 0xffffu) << 16);
-        nmask[r] = static_cast< uint16_t >(ambiguous & 0xffffu);
-        if(L > 16) {
-            bases[pitch + r] = (lo >> 16) | (hi & 0xffff0000u);
-            nmask[pitch + r] = static_cast< uint16_t >(ambiguous >> 16);
+        if(MAX <= 32) {
+            bases[r] = (static_cast< uint32_t >(lo) & 0xffffu) | ((static_cast< uint32_t >(hi) & 0xffffu) << 16);
+            nmask[r] = static_cast< uint16_t >(static_cast< uint32_t >(ambiguous) & 0xffffu);
+            if(L > 16) {
+                bases[pitch + r] = (static_cast< uint32_t >(lo) >> 16) | (static_cast< uint32_t >(hi) & 0xffff0000u);
+                nmask[pitch + r] = static_cast< uint16_t >(static_cast< uint32_t >(ambiguous) >> 16);
+            }
+        } else {
+            #pragma unroll
+            for(int w = 0; w < MAX / 16; ++w) {
+                if(16 * w < L) {
+                    bases[w * pitch + r] = static_cast< uint32_t >((lo >> (16 * w)) & 0xffffu) | (static_cast< uint32_t >((hi >> (16 * w)) & 0xffffu) << 16);
+                    nmask[w * pitch + r] = static_cast< uint16_t >((ambiguous >> (16 * w)) & 0xffffu);
+                }
+            }
         }
         #pragma unroll
-        for(int w = 0; w < PHQ_MAX_NUCLEOTIDES / 4; ++w) {
+        for(int w = 0; w < MAX / 4; ++w) {
             if(4 * w < L) { quality[w * pitch + r] = phred[w]; }
         }
     }
@@ -317,7 +334,12 @@ cudaError_t launch_pack(const PackPlan& plan, long long n_reads, uint32_t* bases
     const int threads = 256;
     const long long blocks = (n_reads + threads - 1) / threads;
     const long long resident = static_cast< long long >(multiprocessor_count) * 8;
-    pack_kernel<<< static_cast< int >(blocks < resident ? blocks : resident), threads, 0, stream >>>(plan, n_reads, bases, nmask, quality, pitch);
+    const int grid = static_cast< int >(blocks < resident ? blocks : resident);
+    if(plan.nucleotide_cardinality > 32) {
+        pack_kernel< PHQ_MAX_NUCLEOTIDES ><<< grid, threads, 0, stream >>>(plan, n_reads, bases, nmask, quality, pitch);
+    } else {
+        pack_kernel< 32 ><<< grid, threads, 0, stream >>>(plan, n_reads, bases, nmask, quality, pitch);
+    }
     return cudaGetLastError();
 }
 
