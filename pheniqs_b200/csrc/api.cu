@@ -171,6 +171,19 @@ void assemble_phred(std::vector< double >& table, double& uniform_quality, doubl
     table[PHRED_UNIFORM_FACTOR] = pow(base, uniform_quality);
 }
 
+/* the 2-bit code the barcode tables hold for a BAM base code: A 0, C 1, G 2, T 3 */
+inline uint32_t two_bit_code(uint8_t code) { return code == 1 ? 0u : code == 2 ? 1u : code == 4 ? 2u : 3u; }
+
+/* positions [from, to) of barcode b as low / high bit-planes, position `from` at bit 0 */
+void barcode_planes(const DecoderSpec& d, int32_t b, int32_t from, int32_t to, uint32_t& lo, uint32_t& hi) {
+    lo = 0; hi = 0;
+    for(int32_t j(from); j < to; ++j) {
+        const uint32_t two(two_bit_code(d.barcode[static_cast< size_t >(b) * d.nucleotide_cardinality + j]));
+        lo |= (two & 1u) << (j - from);
+        hi |= (two >> 1) << (j - from);
+    }
+}
+
 void upload_barcodes(phq_handle* h, size_t k) {
     const DecoderSpec& d(h->chain[k]);
     if(d.nucleotide_cardinality > LONG_NUCLEOTIDES) {
@@ -180,17 +193,8 @@ void upload_barcodes(phq_handle* h, size_t k) {
         for(int32_t b(0); b < d.barcode_cardinality; ++b) {
             LongBarcodeEntry e;
             memset(&e, 0, sizeof(e));
-            for(int32_t j(0); j < d.nucleotide_cardinality; ++j) {
-                const uint8_t code(d.barcode[static_cast< size_t >(b) * d.nucleotide_cardinality + j]);
-                const uint32_t two(code == 1 ? 0u : code == 2 ? 1u : code == 4 ? 2u : 3u);
-                if(j < split) {
-                    e.lo0 |= (two & 1u) << j;
-                    e.hi0 |= (two >> 1) << j;
-                } else {
-                    e.lo1 |= (two & 1u) << (j - split);
-                    e.hi1 |= (two >> 1) << (j - split);
-                }
-            }
+            barcode_planes(d, b, 0, split, e.lo0, e.hi0);
+            barcode_planes(d, b, split, d.nucleotide_cardinality, e.lo1, e.hi1);
             e.prior = d.concentration[b];
             table[b] = e;
         }
@@ -200,13 +204,7 @@ void upload_barcodes(phq_handle* h, size_t k) {
     std::vector< BarcodeEntry > table(static_cast< size_t >(d.barcode_cardinality));
     for(int32_t b(0); b < d.barcode_cardinality; ++b) {
         BarcodeEntry e;
-        e.lo = 0; e.hi = 0;
-        for(int32_t j(0); j < d.nucleotide_cardinality; ++j) {
-            const uint8_t code(d.barcode[static_cast< size_t >(b) * d.nucleotide_cardinality + j]);
-            const uint32_t two(code == 1 ? 0u : code == 2 ? 1u : code == 4 ? 2u : 3u);
-            e.lo |= (two & 1u) << j;
-            e.hi |= (two >> 1) << j;
-        }
+        barcode_planes(d, b, 0, d.nucleotide_cardinality, e.lo, e.hi);
         e.prior = d.concentration[b];
         table[b] = e;
     }
@@ -223,13 +221,8 @@ void upload_fast(phq_handle* h, size_t k) {
     std::vector< FastEntry > table(static_cast< size_t >(d.barcode_cardinality));
     for(int32_t b(0); b < d.barcode_cardinality; ++b) {
         FastEntry e;
-        e.lo = 0; e.hi = 0; e.pad = 0;
-        for(int32_t j(0); j < d.nucleotide_cardinality; ++j) {
-            const uint8_t code(d.barcode[static_cast< size_t >(b) * d.nucleotide_cardinality + j]);
-            const uint32_t two(code == 1 ? 0u : code == 2 ? 1u : code == 4 ? 2u : 3u);
-            e.lo |= (two & 1u) << j;
-            e.hi |= (two >> 1) << j;
-        }
+        e.pad = 0;
+        barcode_planes(d, b, 0, d.nucleotide_cardinality, e.lo, e.hi);
         e.prior = static_cast< float >(d.concentration[b]);
         table[b] = e;
     }
@@ -249,24 +242,15 @@ void upload_grid(phq_handle* h, size_t k) {
     const int32_t split(d.segment_length[0]);
     const int32_t L(d.nucleotide_cardinality);
     if(!grid_shape_supported(split, L)) { return; }
-    auto planes = [&](int32_t b, int32_t from, int32_t to, uint32_t& lo, uint32_t& hi) {
-        lo = 0; hi = 0;
-        for(int32_t j(from); j < to; ++j) {
-            const uint8_t code(d.barcode[static_cast< size_t >(b) * L + j]);
-            const uint32_t two(code == 1 ? 0u : code == 2 ? 1u : code == 4 ? 2u : 3u);
-            lo |= (two & 1u) << (j - from);
-            hi |= (two >> 1) << (j - from);
-        }
-    };
     std::map< std::pair< uint32_t, uint32_t >, std::vector< int32_t > > by_prefix;
     std::map< std::pair< uint32_t, uint32_t >, int32_t > suffix_index;
     std::vector< std::pair< uint32_t, uint32_t > > suffix_word;
     std::vector< int32_t > suffix_of(static_cast< size_t >(d.barcode_cardinality));
     for(int32_t b(0); b < d.barcode_cardinality; ++b) {
         uint32_t lo, hi;
-        planes(b, 0, split, lo, hi);
+        barcode_planes(d, b, 0, split, lo, hi);
         by_prefix[std::make_pair(lo, hi)].push_back(b);
-        planes(b, split, L, lo, hi);
+        barcode_planes(d, b, split, L, lo, hi);
         const auto key(std::make_pair(lo, hi));
         auto found(suffix_index.find(key));
         if(found == suffix_index.end()) {
@@ -363,13 +347,9 @@ void upload_whitelist(phq_handle* h, size_t k) {
         for(int32_t i(0); i < WHITELIST_CHUNK; ++i) {
             const size_t b(c * WHITELIST_CHUNK + static_cast< size_t >(i));
             if(b >= static_cast< size_t >(d.barcode_cardinality)) { break; }      /* padding: no plane bit, prior 0 */
-            uint32_t lo(0), hi(0);
             for(int32_t j(0); j < L; ++j) {
-                const uint8_t code(d.barcode[b * L + j]);
-                const uint32_t two(code == 1 ? 0u : code == 2 ? 1u : code == 4 ? 2u : 3u);
-                lo |= (two & 1u) << j;
-                hi |= (two >> 1) << j;
-                equality[(j * WHITELIST_PLANES + static_cast< int32_t >(two)) * WHITELIST_BLOCKS + (i >> 5)] |= 1u << (i & 31);
+                const int32_t two(static_cast< int32_t >(two_bit_code(d.barcode[b * L + j])));
+                equality[(j * WHITELIST_PLANES + two) * WHITELIST_BLOCKS + (i >> 5)] |= 1u << (i & 31);
             }
             if(d.concentration[b] > largest) { largest = d.concentration[b]; }
         }
@@ -399,8 +379,7 @@ void upload_mdd_tables(phq_handle* h, size_t k) {
         for(int32_t b(0); b < d.barcode_cardinality; ++b) {
             std::vector< uint8_t > w;
             for(int32_t j(d.segment_offset[s]); j < d.segment_offset[s + 1]; ++j) {
-                const uint8_t code(d.barcode[static_cast< size_t >(b) * L + j]);
-                w.push_back(code == 1 ? 0 : code == 2 ? 1 : code == 4 ? 2 : 3);
+                w.push_back(static_cast< uint8_t >(two_bit_code(d.barcode[static_cast< size_t >(b) * L + j])));
             }
             auto found(index.find(w));
             if(found == index.end()) {
@@ -703,6 +682,20 @@ void ensure_slots(phq_handle* h) {
     h->slots_ready = true;
 }
 
+/*  The status of the exception in flight; its message goes where phq_last_error finds it: on the handle, or in the
+    thread's global error without one. Call it from a catch(...) block. */
+int record_error(phq_handle* h) {
+    int status;
+    std::string message;
+    try { throw; }
+    catch(const phq::Error& e) { status = e.code; message = e.what(); }
+    catch(const JsonError& e) { status = PHQ_CONFIGURATION_ERROR; message = std::string("Configuration error : ") + e.what(); }
+    catch(const std::bad_alloc&) { status = PHQ_OUT_OF_MEMORY_ERROR; message = "Out of memory error"; }
+    catch(const std::exception& e) { status = PHQ_UNKNOWN_ERROR; message = e.what(); }
+    (h != NULL ? h->error : global_error) = message;
+    return status;
+}
+
 template < class F > int guarded(phq_handle* h, F body) {
     try {
         if(h == NULL) { throw InternalError("null handle"); }
@@ -710,20 +703,7 @@ template < class F > int guarded(phq_handle* h, F body) {
         PHQ_CUDA(cudaSetDevice(h->device));
         body();
         return PHQ_OK;
-    } catch(const phq::Error& e) {
-        if(h != NULL) { h->error = e.what(); } else { global_error = e.what(); }
-        return e.code;
-    } catch(const JsonError& e) {
-        std::string m(std::string("Configuration error : ") + e.what());
-        if(h != NULL) { h->error = m; } else { global_error = m; }
-        return PHQ_CONFIGURATION_ERROR;
-    } catch(const std::bad_alloc&) {
-        if(h != NULL) { h->error = "Out of memory error"; } else { global_error = "Out of memory error"; }
-        return PHQ_OUT_OF_MEMORY_ERROR;
-    } catch(const std::exception& e) {
-        if(h != NULL) { h->error = e.what(); } else { global_error = e.what(); }
-        return PHQ_UNKNOWN_ERROR;
-    }
+    } catch(...) { return record_error(h); }
 }
 
 /* a handle whose accumulators hold the sums of all ranks must be reset before it accumulates again (phq_collect) */
@@ -742,18 +722,82 @@ void require_compact_range(const phq_handle* h) {
     }
 }
 
+/*  The host-buffer decode calls: reads [0, n_reads) in sub-batches rotating over the staging slots, so that one
+    sub-batch's copies overlap another's kernels. On the slot's stream, per sub-batch: qcfail in, stage_tiles (fills
+    the slot's tile buffers of every tiled decoder), the chain, after_chain, then results and qcfail out. Both steps
+    take (slot, first read, reads, pitch of the slot buffers); stage_tiles also the device tiles, after_chain the
+    device results. */
+template < class StageTiles, class AfterChain >
+void decode_staged(phq_handle* h, int64_t n_reads, bool tags, const uint8_t* qcfail_in, phq_result* const* results,
+                   phq_compact_result* const* compact, uint8_t* qcfail_out, StageTiles stage_tiles, AfterChain after_chain) {
+    refuse_collected(h);
+    if(compact != NULL) { require_compact_range(h); }
+    ensure_slots(h);
+    const size_t n_decoders(h->chain.size());
+    /* compact results take the 8-byte form on the device, unless the tag kernel reads them: it reads the 16-byte form */
+    const bool compact_on_device(compact != NULL && !tags);
+    const long long sub(n_reads < h->sub_batch_reads ? (n_reads > 0 ? n_reads : 1) : h->sub_batch_reads);
+    int turn(0);
+    for(long long begin(0); begin < n_reads; begin += sub, ++turn) {
+        const long long count((n_reads - begin) < sub ? (n_reads - begin) : sub);
+        StagingSlot& s(h->slot[turn % STAGING_SLOTS]);
+        if(turn >= STAGING_SLOTS) { PHQ_CUDA(cudaEventSynchronize(s.done)); }
+        s.qcfail.reserve(static_cast< size_t >(sub));
+        if(qcfail_in != NULL) { PHQ_CUDA(cudaMemcpyAsync(s.qcfail.pointer, qcfail_in + begin, static_cast< size_t >(count), cudaMemcpyHostToDevice, s.stream)); }
+        else { PHQ_CUDA(cudaMemsetAsync(s.qcfail.pointer, 0, static_cast< size_t >(count), s.stream)); }
+        std::vector< phq_tile > device_tiles(n_decoders);
+        std::vector< phq_result* > device_results(n_decoders, static_cast< phq_result* >(NULL));
+        std::vector< phq_compact_result* > device_compact(n_decoders, static_cast< phq_compact_result* >(NULL));
+        for(size_t k(0); k < n_decoders; ++k) {
+            const DecoderSpec& d(h->chain[k]);
+            if(d.tiled()) {
+                s.bases[k].reserve(static_cast< size_t >(sub) * d.word_cardinality());
+                s.nmask[k].reserve(static_cast< size_t >(sub) * d.word_cardinality());
+                s.quality[k].reserve(static_cast< size_t >(sub) * d.quality_word_cardinality());
+                device_tiles[k].bases = s.bases[k].pointer;
+                device_tiles[k].nmask = s.nmask[k].pointer;
+                device_tiles[k].quality = s.quality[k].pointer;
+                device_tiles[k].pitch = sub;
+            }
+            if((results != NULL && results[k] != NULL) || (compact != NULL && compact[k] != NULL) || (tags && d.tiled())) {
+                /* the staging buffer is sized for the 16-byte form and reused for the 8-byte one */
+                s.results[k].reserve(static_cast< size_t >(sub));
+                if(compact_on_device) { device_compact[k] = reinterpret_cast< phq_compact_result* >(s.results[k].pointer); }
+                else { device_results[k] = s.results[k].pointer; }
+            }
+        }
+        stage_tiles(s, begin, count, sub, device_tiles.data());
+        launch_chain(h, count, device_tiles.data(), s.qcfail.pointer, device_results.data(), device_compact.data(), s.tie_list, s.stream);
+        after_chain(s, begin, count, sub, device_results.data());
+        for(size_t k(0); k < n_decoders; ++k) {
+            if(device_results[k] != NULL && results != NULL && results[k] != NULL) {
+                PHQ_CUDA(cudaMemcpyAsync(results[k] + begin, device_results[k], static_cast< size_t >(count) * sizeof(phq_result), cudaMemcpyDeviceToHost, s.stream));
+            }
+            if(device_compact[k] != NULL) {
+                PHQ_CUDA(cudaMemcpyAsync(compact[k] + begin, device_compact[k], static_cast< size_t >(count) * sizeof(phq_compact_result), cudaMemcpyDeviceToHost, s.stream));
+            }
+        }
+        if(qcfail_out != NULL) { PHQ_CUDA(cudaMemcpyAsync(qcfail_out + begin, s.qcfail.pointer, static_cast< size_t >(count), cudaMemcpyDeviceToHost, s.stream)); }
+        PHQ_CUDA(cudaEventRecord(s.done, s.stream));
+    }
+    for(int i(0); i < STAGING_SLOTS && i < turn; ++i) { PHQ_CUDA(cudaStreamSynchronize(h->slot[i].stream)); }
+}
+
 /* for entry points that are pure host work and therefore also serve host-only handles */
 template < class F > int guarded_host(phq_handle* h, F body) {
     try {
         if(h == NULL) { throw InternalError("null handle"); }
         body();
         return PHQ_OK;
-    } catch(const phq::Error& e) { h != NULL ? h->error = e.what() : global_error = e.what(); return e.code; }
-    catch(const JsonError& e) {
-        std::string m(std::string("Configuration error : ") + e.what());
-        h != NULL ? h->error = m : global_error = m;
-        return PHQ_CONFIGURATION_ERROR;
-    } catch(const std::exception& e) { h != NULL ? h->error = e.what() : global_error = e.what(); return PHQ_UNKNOWN_ERROR; }
+    } catch(...) { return record_error(h); }
+}
+
+/* a malloc'd copy the caller releases with phq_free */
+char* duplicate(const std::string& text) {
+    char* out(static_cast< char* >(malloc(text.size() + 1)));
+    if(out == NULL) { throw phq::Error(PHQ_OUT_OF_MEMORY_ERROR, "Out of memory error"); }
+    memcpy(out, text.c_str(), text.size() + 1);
+    return out;
 }
 
 }   /* namespace */
@@ -768,15 +812,9 @@ int phq_compile_job(const char* job_json, char** compiled_json) {
     try {
         if(job_json == NULL || compiled_json == NULL) { throw InternalError("null argument"); }
         Json compiled(compile_job(Json::parse(job_json)));
-        std::string text(compiled.dump(-1, 4));     /* shortest round-trip decimals: priors must survive the text form bit for bit */
-        char* out(static_cast< char* >(malloc(text.size() + 1)));
-        if(out == NULL) { throw phq::Error(PHQ_OUT_OF_MEMORY_ERROR, "Out of memory error"); }
-        memcpy(out, text.c_str(), text.size() + 1);
-        *compiled_json = out;
+        *compiled_json = duplicate(compiled.dump(-1, 4));     /* shortest round-trip decimals: priors must survive the text form bit for bit */
         return PHQ_OK;
-    } catch(const phq::Error& e) { global_error = e.what(); return e.code; }
-    catch(const JsonError& e) { global_error = std::string("Configuration error : ") + e.what(); return PHQ_CONFIGURATION_ERROR; }
-    catch(const std::exception& e) { global_error = e.what(); return PHQ_UNKNOWN_ERROR; }
+    } catch(...) { return record_error(NULL); }
 }
 
 int phq_load_job(const char* path, char** job_json) {
@@ -785,14 +823,9 @@ int phq_load_job(const char* path, char** job_json) {
     try {
         std::set< std::string > visited;
         const Json job(load_job_with_import(path, visited));
-        const std::string text(job.dump(-1, 4));
-        *job_json = static_cast< char* >(malloc(text.size() + 1));
-        if(*job_json == NULL) { global_error = "Out of memory error"; return PHQ_OUT_OF_MEMORY_ERROR; }
-        memcpy(*job_json, text.c_str(), text.size() + 1);
+        *job_json = duplicate(job.dump(-1, 4));
         return PHQ_OK;
-    } catch(const phq::Error& e) { global_error = e.what(); return e.code; }
-    catch(const JsonError& e) { global_error = std::string("Configuration error : ") + e.what(); return PHQ_CONFIGURATION_ERROR; }
-    catch(const std::exception& e) { global_error = e.what(); return PHQ_UNKNOWN_ERROR; }
+    } catch(...) { return record_error(NULL); }
 }
 
 int phq_create(const char* compiled_job_json, int device, phq_handle** handle) {
@@ -901,10 +934,11 @@ int phq_create(const char* compiled_job_json, int device, phq_handle** handle) {
         PHQ_CUDA(prepare_kernels(h->geometry));
         *handle = h;
         return PHQ_OK;
-    } catch(const phq::Error& e) { global_error = e.what(); destroy(h); return e.code; }
-    catch(const JsonError& e) { global_error = std::string("Configuration error : ") + e.what(); destroy(h); return PHQ_CONFIGURATION_ERROR; }
-    catch(const std::bad_alloc&) { global_error = "Out of memory error"; destroy(h); return PHQ_OUT_OF_MEMORY_ERROR; }
-    catch(const std::exception& e) { global_error = e.what(); destroy(h); return PHQ_UNKNOWN_ERROR; }
+    } catch(...) {
+        const int status(record_error(NULL));
+        destroy(h);
+        return status;
+    }
 }
 
 void phq_destroy(phq_handle* handle) { destroy(handle); }
@@ -934,9 +968,8 @@ int phq_decoder_describe(const phq_handle* handle, int decoder, phq_decoder_info
 int phq_pack(phq_handle* handle, int64_t n_reads, int32_t n_input_segments,
              const uint8_t* const* code, const uint8_t* const* quality, const int64_t* const* offset,
              phq_tile* tiles) {
-    phq_handle* h(handle);
-    try {
-        if(h == NULL) { throw InternalError("null handle"); }
+    return guarded_host(handle, [&]() {
+        phq_handle* h(handle);
         if(n_reads < 0 || tiles == NULL) { throw InternalError("illegal argument"); }
         for(size_t k(0); k < h->chain.size(); ++k) {
             const DecoderSpec& d(h->chain[k]);
@@ -1104,9 +1137,7 @@ int phq_pack(phq_handle* handle, int64_t n_reads, int32_t n_input_segments,
             }
             tile.quality_bits = wanted;
         }
-        return PHQ_OK;
-    } catch(const phq::Error& e) { if(h != NULL) { h->error = e.what(); } else { global_error = e.what(); } return e.code; }
-    catch(const std::exception& e) { if(h != NULL) { h->error = e.what(); } else { global_error = e.what(); } return PHQ_UNKNOWN_ERROR; }
+    });
 }
 
 static int decode_device(phq_handle* handle, int64_t n_reads, const phq_tile* device_tiles, uint8_t* device_qcfail,
@@ -1138,67 +1169,26 @@ static int decode_host(phq_handle* handle, int64_t n_reads, const phq_tile* tile
     return guarded(handle, [&]() {
         phq_handle* h(handle);
         if(n_reads < 0) { throw InternalError("illegal read count"); }
-        refuse_collected(h);
-        if(compact != NULL) { require_compact_range(h); }
-        ensure_slots(h);
-        const size_t n_decoders(h->chain.size());
-        const long long sub(n_reads < h->sub_batch_reads ? (n_reads > 0 ? n_reads : 1) : h->sub_batch_reads);
-        int turn(0);
-        for(long long begin(0); begin < n_reads; begin += sub, ++turn) {
-            const long long count((n_reads - begin) < sub ? (n_reads - begin) : sub);
-            StagingSlot& s(h->slot[turn % STAGING_SLOTS]);
-            if(turn >= STAGING_SLOTS) { PHQ_CUDA(cudaEventSynchronize(s.done)); }
-            std::vector< phq_tile > device_tiles(n_decoders);
-            std::vector< phq_result* > device_results(n_decoders, static_cast< phq_result* >(NULL));
-            std::vector< phq_compact_result* > device_compact(n_decoders, static_cast< phq_compact_result* >(NULL));
-            s.qcfail.reserve(static_cast< size_t >(sub));
-            if(qcfail_in != NULL) { PHQ_CUDA(cudaMemcpyAsync(s.qcfail.pointer, qcfail_in + begin, static_cast< size_t >(count), cudaMemcpyHostToDevice, s.stream)); }
-            else { PHQ_CUDA(cudaMemsetAsync(s.qcfail.pointer, 0, static_cast< size_t >(count), s.stream)); }
-            for(size_t k(0); k < n_decoders; ++k) {
+        auto copy_tiles = [&](StagingSlot& s, long long begin, long long count, long long sub, phq_tile* device_tiles) {
+            for(size_t k(0); k < h->chain.size(); ++k) {
                 const DecoderSpec& d(h->chain[k]);
-                memset(&device_tiles[k], 0, sizeof(phq_tile));
-                if(d.tiled()) {
-                    if(tiles == NULL || tiles[k].bases == NULL) { throw InternalError("decoder " + std::to_string(k) + " needs a tile"); }
-                    const int32_t words(d.word_cardinality());
-                    const int32_t bits(tiles[k].quality_bits == 0 ? 8 : tiles[k].quality_bits);
-                    /* only the rows the chosen quality form occupies travel */
-                    const int32_t quality_words((d.nucleotide_cardinality * bits + 31) / 32);
-                    s.bases[k].reserve(static_cast< size_t >(sub) * words);
-                    s.nmask[k].reserve(static_cast< size_t >(sub) * words);
-                    s.quality[k].reserve(static_cast< size_t >(sub) * d.quality_word_cardinality());
-                    PHQ_CUDA(cudaMemcpy2DAsync(s.bases[k].pointer, static_cast< size_t >(sub) * 4, tiles[k].bases + begin, static_cast< size_t >(tiles[k].pitch) * 4,
-                                               static_cast< size_t >(count) * 4, words, cudaMemcpyHostToDevice, s.stream));
-                    PHQ_CUDA(cudaMemcpy2DAsync(s.nmask[k].pointer, static_cast< size_t >(sub) * 2, tiles[k].nmask + begin, static_cast< size_t >(tiles[k].pitch) * 2,
-                                               static_cast< size_t >(count) * 2, words, cudaMemcpyHostToDevice, s.stream));
-                    PHQ_CUDA(cudaMemcpy2DAsync(s.quality[k].pointer, static_cast< size_t >(sub) * 4, tiles[k].quality + begin, static_cast< size_t >(tiles[k].pitch) * 4,
-                                               static_cast< size_t >(count) * 4, quality_words, cudaMemcpyHostToDevice, s.stream));
-                    device_tiles[k] = tiles[k];
-                    device_tiles[k].bases = s.bases[k].pointer;
-                    device_tiles[k].nmask = s.nmask[k].pointer;
-                    device_tiles[k].quality = s.quality[k].pointer;
-                    device_tiles[k].pitch = sub;
-                }
-                const bool wanted((results != NULL && results[k] != NULL) || (compact != NULL && compact[k] != NULL));
-                if(wanted) {
-                    /* the staging buffer is sized for the 16-byte form and reused for the 8-byte one */
-                    s.results[k].reserve(static_cast< size_t >(sub));
-                    if(compact != NULL) { device_compact[k] = reinterpret_cast< phq_compact_result* >(s.results[k].pointer); }
-                    else { device_results[k] = s.results[k].pointer; }
-                }
+                if(!d.tiled()) { continue; }
+                if(tiles == NULL || tiles[k].bases == NULL) { throw InternalError("decoder " + std::to_string(k) + " needs a tile"); }
+                const int32_t words(d.word_cardinality());
+                const int32_t bits(tiles[k].quality_bits == 0 ? 8 : tiles[k].quality_bits);
+                /* only the rows the chosen quality form occupies travel */
+                const int32_t quality_words((d.nucleotide_cardinality * bits + 31) / 32);
+                PHQ_CUDA(cudaMemcpy2DAsync(s.bases[k].pointer, static_cast< size_t >(sub) * 4, tiles[k].bases + begin, static_cast< size_t >(tiles[k].pitch) * 4,
+                                           static_cast< size_t >(count) * 4, words, cudaMemcpyHostToDevice, s.stream));
+                PHQ_CUDA(cudaMemcpy2DAsync(s.nmask[k].pointer, static_cast< size_t >(sub) * 2, tiles[k].nmask + begin, static_cast< size_t >(tiles[k].pitch) * 2,
+                                           static_cast< size_t >(count) * 2, words, cudaMemcpyHostToDevice, s.stream));
+                PHQ_CUDA(cudaMemcpy2DAsync(s.quality[k].pointer, static_cast< size_t >(sub) * 4, tiles[k].quality + begin, static_cast< size_t >(tiles[k].pitch) * 4,
+                                           static_cast< size_t >(count) * 4, quality_words, cudaMemcpyHostToDevice, s.stream));
+                device_tiles[k].quality_bits = tiles[k].quality_bits;
+                memcpy(device_tiles[k].quality_codebook, tiles[k].quality_codebook, sizeof(tiles[k].quality_codebook));
             }
-            launch_chain(h, count, device_tiles.data(), s.qcfail.pointer, compact != NULL ? NULL : device_results.data(), compact != NULL ? device_compact.data() : NULL, s.tie_list, s.stream);
-            for(size_t k(0); k < n_decoders; ++k) {
-                if(device_results[k] != NULL) {
-                    PHQ_CUDA(cudaMemcpyAsync(results[k] + begin, device_results[k], static_cast< size_t >(count) * sizeof(phq_result), cudaMemcpyDeviceToHost, s.stream));
-                }
-                if(device_compact[k] != NULL) {
-                    PHQ_CUDA(cudaMemcpyAsync(compact[k] + begin, device_compact[k], static_cast< size_t >(count) * sizeof(phq_compact_result), cudaMemcpyDeviceToHost, s.stream));
-                }
-            }
-            if(qcfail_out != NULL) { PHQ_CUDA(cudaMemcpyAsync(qcfail_out + begin, s.qcfail.pointer, static_cast< size_t >(count), cudaMemcpyDeviceToHost, s.stream)); }
-            PHQ_CUDA(cudaEventRecord(s.done, s.stream));
-        }
-        for(int i(0); i < STAGING_SLOTS && i < turn; ++i) { PHQ_CUDA(cudaStreamSynchronize(h->slot[i].stream)); }
+        };
+        decode_staged(h, n_reads, false, qcfail_in, results, compact, qcfail_out, copy_tiles, [](auto&&...) {});
     });
 }
 int phq_decode_batch(phq_handle* handle, int64_t n_reads, const phq_tile* tiles,
@@ -1342,6 +1332,14 @@ void ensure_tags(phq_handle* h) {
     h->tags_ready = true;
 }
 
+/* a token in the form the pack and tag kernels read */
+PackToken pack_token(const TransformSpec& t) {
+    PackToken to;
+    to.input_segment = t.input_segment_index; to.start = t.start; to.end = t.end; to.end_terminated = t.end_terminated ? 1 : 0;
+    to.output_segment = t.output_segment_index; to.reverse_complement = t.reverse_complement ? 1 : 0;
+    return to;
+}
+
 int decode_raw(phq_handle* handle, int64_t n_reads, int32_t n_input_segments, const phq_raw_segment* segments, int32_t phred_offset,
                const uint8_t* qcfail_in, phq_result* const* results, phq_compact_result* const* compact, uint8_t* qcfail_out,
                uint8_t* aux = NULL, int32_t* aux_length = NULL, int32_t aux_stride = 0, bool bam_input = false) {
@@ -1356,9 +1354,6 @@ int decode_raw(phq_handle* handle, int64_t n_reads, int32_t n_input_segments, co
         }
         if(n_reads < 0 || n_input_segments < 0 || (n_input_segments > 0 && segments == NULL)) { throw InternalError("illegal argument"); }
         if(n_input_segments > PACK_MAX_INPUT_SEGMENTS) { throw ConfigurationError("more than " + std::to_string(PACK_MAX_INPUT_SEGMENTS) + " input segments are not supported on this path"); }
-        refuse_collected(h);
-        if(compact != NULL) { require_compact_range(h); }
-        ensure_slots(h);
         const size_t n_decoders(h->chain.size());
         std::vector< bool > used(static_cast< size_t >(n_input_segments), false);
         for(size_t k(0); k < n_decoders; ++k) {
@@ -1378,21 +1373,12 @@ int decode_raw(phq_handle* handle, int64_t n_reads, int32_t n_input_segments, co
                 throw InternalError("input segment " + std::to_string(i) + " has no bytes");
             }
         }
-        const long long sub(n_reads < h->sub_batch_reads ? (n_reads > 0 ? n_reads : 1) : h->sub_batch_reads);
-        int turn(0);
-        for(long long begin(0); begin < n_reads; begin += sub, ++turn) {
-            const long long count((n_reads - begin) < sub ? (n_reads - begin) : sub);
-            StagingSlot& s(h->slot[turn % STAGING_SLOTS]);
-            if(turn >= STAGING_SLOTS) { PHQ_CUDA(cudaEventSynchronize(s.done)); }
+        /* the bytes of the current sub-batch's reads, as they sit in the feed buffers: filled by upload_and_pack, read by the tag step */
+        RawSegmentView view[PACK_MAX_INPUT_SEGMENTS];
+        auto upload_and_pack = [&](StagingSlot& s, long long begin, long long count, long long sub, phq_tile*) {
             s.raw_sequence.resize(static_cast< size_t >(n_input_segments));
             s.raw_quality.resize(static_cast< size_t >(n_input_segments));
             s.raw_offset.resize(static_cast< size_t >(n_input_segments));
-            s.qcfail.reserve(static_cast< size_t >(sub));
-            if(qcfail_in != NULL) { PHQ_CUDA(cudaMemcpyAsync(s.qcfail.pointer, qcfail_in + begin, static_cast< size_t >(count), cudaMemcpyHostToDevice, s.stream)); }
-            else { PHQ_CUDA(cudaMemsetAsync(s.qcfail.pointer, 0, static_cast< size_t >(count), s.stream)); }
-
-            /* the bytes of this sub-batch's reads, as they sit in the feed buffers */
-            RawSegmentView view[PACK_MAX_INPUT_SEGMENTS];
             memset(view, 0, sizeof(view));
             for(int32_t i(0); i < n_input_segments; ++i) {
                 if(!used[i]) { continue; }
@@ -1418,103 +1404,61 @@ int decode_raw(phq_handle* handle, int64_t n_reads, int32_t n_input_segments, co
                     view[i].first = begin;      /* r * length is absolute like the offsets */
                 }
             }
-
-            std::vector< phq_tile > device_tiles(n_decoders);
-            std::vector< phq_result* > device_results(n_decoders, static_cast< phq_result* >(NULL));
-            std::vector< phq_compact_result* > device_compact(n_decoders, static_cast< phq_compact_result* >(NULL));
             for(size_t k(0); k < n_decoders; ++k) {
                 const DecoderSpec& d(h->chain[k]);
-                memset(&device_tiles[k], 0, sizeof(phq_tile));
-                if(d.tiled()) {
-                    s.bases[k].reserve(static_cast< size_t >(sub) * d.word_cardinality());
-                    s.nmask[k].reserve(static_cast< size_t >(sub) * d.word_cardinality());
-                    s.quality[k].reserve(static_cast< size_t >(sub) * d.quality_word_cardinality());
-                    PackPlan plan;
-                    memset(&plan, 0, sizeof(plan));
-                    plan.token_cardinality = static_cast< int32_t >(d.transform.size());
-                    plan.segment_cardinality = d.segment_cardinality;
-                    plan.nucleotide_cardinality = d.nucleotide_cardinality;
-                    plan.stale_semantics = d.algorithm == PHQ_PAMLD ? 1 : 0;
-                    plan.phred_offset = phred_offset;
-                    plan.bam_input = bam_input ? 1 : 0;
-                    for(int32_t i(0); i <= d.segment_cardinality; ++i) { plan.segment_offset[i] = d.segment_offset[i]; }
-                    for(size_t i(0); i < d.transform.size(); ++i) {
-                        const TransformSpec& t(d.transform[i]);
-                        PackToken& to(plan.token[i]);
-                        to.input_segment = t.input_segment_index; to.start = t.start; to.end = t.end; to.end_terminated = t.end_terminated ? 1 : 0;
-                        to.output_segment = t.output_segment_index; to.reverse_complement = t.reverse_complement ? 1 : 0;
-                    }
-                    memcpy(plan.input, view, sizeof(view));
-                    /* the kernel indexes reads from 0: move the views to this sub-batch */
-                    for(int32_t i(0); i < n_input_segments; ++i) { if(plan.input[i].offset == NULL) { plan.input[i].first = begin; } }
-                    if(plan.stale_semantics) {
-                        const RawReader reader{ d, segments, phred_offset, bam_input };
-                        reader.state_after(begin - 1, h->scratch[k], plan.carry_code, plan.carry_quality);
-                    }
-                    PHQ_CUDA(launch_pack(plan, count, s.bases[k].pointer, s.nmask[k].pointer, s.quality[k].pointer, sub, h->geometry.multiprocessor_count, s.stream));
-                    h->kernel_launches += 1;
-                    device_tiles[k].bases = s.bases[k].pointer;
-                    device_tiles[k].nmask = s.nmask[k].pointer;
-                    device_tiles[k].quality = s.quality[k].pointer;
-                    device_tiles[k].pitch = sub;
-                    device_tiles[k].quality_bits = 8;
-                }
-                const bool wanted((results != NULL && results[k] != NULL) || (compact != NULL && compact[k] != NULL) || (tags && d.tiled()));
-                if(wanted) {
-                    s.results[k].reserve(static_cast< size_t >(sub));
-                    if(compact != NULL && !tags) { device_compact[k] = reinterpret_cast< phq_compact_result* >(s.results[k].pointer); }
-                    else { device_results[k] = s.results[k].pointer; }
-                }
-            }
-            launch_chain(h, count, device_tiles.data(), s.qcfail.pointer, (compact != NULL && !tags) ? NULL : device_results.data(), (compact != NULL && !tags) ? device_compact.data() : NULL, s.tie_list, s.stream);
-            if(tags) {
-                TagPlan plan;
+                if(!d.tiled()) { continue; }
+                PackPlan plan;
                 memset(&plan, 0, sizeof(plan));
-                plan.decoder_cardinality = static_cast< int32_t >(n_decoders);
+                plan.token_cardinality = static_cast< int32_t >(d.transform.size());
+                plan.segment_cardinality = d.segment_cardinality;
+                plan.nucleotide_cardinality = d.nucleotide_cardinality;
+                plan.stale_semantics = d.algorithm == PHQ_PAMLD ? 1 : 0;
                 plan.phred_offset = phred_offset;
                 plan.bam_input = bam_input ? 1 : 0;
-                plan.stride = aux_stride;
-                plan.read_group_text = h->device_read_group_text;
-                plan.read_group_offset = h->device_read_group_offset;
+                for(int32_t i(0); i <= d.segment_cardinality; ++i) { plan.segment_offset[i] = d.segment_offset[i]; }
+                for(size_t i(0); i < d.transform.size(); ++i) { plan.token[i] = pack_token(d.transform[i]); }
                 memcpy(plan.input, view, sizeof(view));
-                for(int32_t i(0); i < n_input_segments; ++i) { if(plan.input[i].offset == NULL) { plan.input[i].first = begin; } }
-                for(size_t k(0); k < n_decoders; ++k) {
-                    const DecoderSpec& d(h->chain[k]);
-                    TagDecoder& to(plan.decoder[k]);
-                    to.topic = d.topic;
-                    to.algorithm = d.algorithm;
-                    to.corrected_quality = d.corrected_quality;
-                    to.token_cardinality = static_cast< int32_t >(d.transform.size());
-                    to.segment_cardinality = d.transform.empty() ? 0 : d.segment_cardinality;
-                    to.nucleotide_cardinality = d.nucleotide_cardinality;
-                    for(int32_t i(0); i <= d.segment_cardinality && i <= PHQ_MAX_SEGMENTS && !d.transform.empty(); ++i) { to.segment_offset[i] = d.segment_offset[i]; }
-                    for(size_t i(0); i < d.transform.size(); ++i) {
-                        const TransformSpec& t(d.transform[i]);
-                        PackToken& token(to.token[i]);
-                        token.input_segment = t.input_segment_index; token.start = t.start; token.end = t.end; token.end_terminated = t.end_terminated ? 1 : 0;
-                        token.output_segment = t.output_segment_index; token.reverse_complement = t.reverse_complement ? 1 : 0;
-                    }
-                    to.results = d.tiled() ? device_results[k] : NULL;
-                    to.barcode_code = h->device_barcode_code[k];
+                if(plan.stale_semantics) {
+                    const RawReader reader{ d, segments, phred_offset, bam_input };
+                    reader.state_after(begin - 1, h->scratch[k], plan.carry_code, plan.carry_quality);
                 }
-                s.aux.reserve(static_cast< size_t >(sub) * aux_stride);
-                s.aux_length.reserve(static_cast< size_t >(sub));
-                PHQ_CUDA(launch_tags(plan, count, s.aux.pointer, s.aux_length.pointer, h->geometry.multiprocessor_count, s.stream));
+                PHQ_CUDA(launch_pack(plan, count, s.bases[k].pointer, s.nmask[k].pointer, s.quality[k].pointer, sub, h->geometry.multiprocessor_count, s.stream));
                 h->kernel_launches += 1;
-                PHQ_CUDA(cudaMemcpyAsync(aux + begin * aux_stride, s.aux.pointer, static_cast< size_t >(count) * aux_stride, cudaMemcpyDeviceToHost, s.stream));
-                PHQ_CUDA(cudaMemcpyAsync(aux_length + begin, s.aux_length.pointer, static_cast< size_t >(count) * sizeof(int32_t), cudaMemcpyDeviceToHost, s.stream));
             }
+        };
+        auto synthesize_tags = [&](StagingSlot& s, long long begin, long long count, long long sub, phq_result* const* device_results) {
+            if(!tags) { return; }
+            TagPlan plan;
+            memset(&plan, 0, sizeof(plan));
+            plan.decoder_cardinality = static_cast< int32_t >(n_decoders);
+            plan.phred_offset = phred_offset;
+            plan.bam_input = bam_input ? 1 : 0;
+            plan.stride = aux_stride;
+            plan.read_group_text = h->device_read_group_text;
+            plan.read_group_offset = h->device_read_group_offset;
+            memcpy(plan.input, view, sizeof(view));
             for(size_t k(0); k < n_decoders; ++k) {
-                if(device_results[k] != NULL && results != NULL && results[k] != NULL) {
-                    PHQ_CUDA(cudaMemcpyAsync(results[k] + begin, device_results[k], static_cast< size_t >(count) * sizeof(phq_result), cudaMemcpyDeviceToHost, s.stream));
-                }
-                if(device_compact[k] != NULL) {
-                    PHQ_CUDA(cudaMemcpyAsync(compact[k] + begin, device_compact[k], static_cast< size_t >(count) * sizeof(phq_compact_result), cudaMemcpyDeviceToHost, s.stream));
-                }
+                const DecoderSpec& d(h->chain[k]);
+                TagDecoder& to(plan.decoder[k]);
+                to.topic = d.topic;
+                to.algorithm = d.algorithm;
+                to.corrected_quality = d.corrected_quality;
+                to.token_cardinality = static_cast< int32_t >(d.transform.size());
+                to.segment_cardinality = d.transform.empty() ? 0 : d.segment_cardinality;
+                to.nucleotide_cardinality = d.nucleotide_cardinality;
+                for(int32_t i(0); i <= d.segment_cardinality && i <= PHQ_MAX_SEGMENTS && !d.transform.empty(); ++i) { to.segment_offset[i] = d.segment_offset[i]; }
+                for(size_t i(0); i < d.transform.size(); ++i) { to.token[i] = pack_token(d.transform[i]); }
+                to.results = d.tiled() ? device_results[k] : NULL;
+                to.barcode_code = h->device_barcode_code[k];
             }
-            if(qcfail_out != NULL) { PHQ_CUDA(cudaMemcpyAsync(qcfail_out + begin, s.qcfail.pointer, static_cast< size_t >(count), cudaMemcpyDeviceToHost, s.stream)); }
-            PHQ_CUDA(cudaEventRecord(s.done, s.stream));
-        }
+            s.aux.reserve(static_cast< size_t >(sub) * aux_stride);
+            s.aux_length.reserve(static_cast< size_t >(sub));
+            PHQ_CUDA(launch_tags(plan, count, s.aux.pointer, s.aux_length.pointer, h->geometry.multiprocessor_count, s.stream));
+            h->kernel_launches += 1;
+            PHQ_CUDA(cudaMemcpyAsync(aux + begin * aux_stride, s.aux.pointer, static_cast< size_t >(count) * aux_stride, cudaMemcpyDeviceToHost, s.stream));
+            PHQ_CUDA(cudaMemcpyAsync(aux_length + begin, s.aux_length.pointer, static_cast< size_t >(count) * sizeof(int32_t), cudaMemcpyDeviceToHost, s.stream));
+        };
+        decode_staged(h, n_reads, tags, qcfail_in, results, compact, qcfail_out, upload_and_pack, synthesize_tags);
         /* leave the Observations as a single reference thread would: later calls (raw or phq_pack) continue from here */
         for(size_t k(0); k < n_decoders && n_reads > 0; ++k) {
             const DecoderSpec& d(h->chain[k]);
@@ -1529,7 +1473,6 @@ int decode_raw(phq_handle* handle, int64_t n_reads, int32_t n_input_segments, co
                 }
             }
         }
-        for(int i(0); i < STAGING_SLOTS && i < turn; ++i) { PHQ_CUDA(cudaStreamSynchronize(h->slot[i].stream)); }
     });
 }
 
@@ -1734,8 +1677,7 @@ const NcclLibrary& nccl() {
 
 template < class F > int guarded_global(F body) {
     try { body(); return PHQ_OK; }
-    catch(const phq::Error& e) { global_error = e.what(); return e.code; }
-    catch(const std::exception& e) { global_error = e.what(); return PHQ_UNKNOWN_ERROR; }
+    catch(...) { return record_error(NULL); }
 }
 
 }   /* namespace */
@@ -1800,15 +1742,6 @@ int phq_statistics(phq_handle* handle, uint64_t* kernel_launches, uint64_t* exac
 }
 
 /* ------------------------------------------------------------------ report and prior adjusted job (report.hpp) */
-namespace {
-char* duplicate(const std::string& text) {
-    char* out(static_cast< char* >(malloc(text.size() + 1)));
-    if(out == NULL) { throw phq::Error(PHQ_OUT_OF_MEMORY_ERROR, "Out of memory error"); }
-    memcpy(out, text.c_str(), text.size() + 1);
-    return out;
-}
-}
-
 int phq_encode_report(phq_handle* handle, const uint64_t* const* u64_tables, const double* const* f64_tables, uint64_t count, uint64_t pf_count,
                       uint64_t incoming_count, uint64_t incoming_pf_count, int precision, char** report_json) {
     return guarded_host(handle, [&]() {
@@ -1851,9 +1784,7 @@ int phq_adjust_job(const char* job_json, const char* report_json, int precision,
         adjusted.sort_keys();
         *adjusted_json = duplicate(adjusted.dump(precision, 4));
         return PHQ_OK;
-    } catch(const phq::Error& e) { global_error = e.what(); return e.code; }
-    catch(const JsonError& e) { global_error = std::string("Configuration error : ") + e.what(); return PHQ_CONFIGURATION_ERROR; }
-    catch(const std::exception& e) { global_error = e.what(); return PHQ_UNKNOWN_ERROR; }
+    } catch(...) { return record_error(NULL); }
 }
 
 int phq_reference_power(phq_handle* handle, int64_t n, const double* sigma, double* power) {

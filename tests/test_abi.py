@@ -270,3 +270,41 @@ def test_threaded_pack_equals_the_sequential_one(short, monkeypatch):
             continue
         assert x.quality_bits == y.quality_bits and bytes(x.quality_codebook) == bytes(y.quality_codebook)
         assert np.array_equal(x.bases, y.bases) and np.array_equal(x.nmask, y.nmask) and np.array_equal(x.quality, y.quality)
+
+
+def test_host_entry_points_report_status_and_message():
+    """The status and message of the entry points that need no device, read where phq_last_error finds them."""
+    lib = binding.library()
+    out = C.c_void_p(1)
+
+    def global_error():
+        return lib.phq_last_global_error().decode()
+
+    assert lib.phq_compile_job(b"{ not json", C.byref(out)) == binding.PHQ_CONFIGURATION_ERROR
+    assert global_error().startswith("Configuration error : ")
+    assert lib.phq_compile_job(None, C.byref(out)) == binding.PHQ_INTERNAL_ERROR
+    assert global_error() == "Internal error : null argument"
+
+    job = json.dumps(compile_job(workload.load("c1")["job"])).encode()
+    assert lib.phq_adjust_job(job, b"{ not json", 6, C.byref(out)) == binding.PHQ_CONFIGURATION_ERROR
+    assert global_error().startswith("Configuration error : ")
+
+    assert lib.phq_load_job(os.path.join(ROOT, "no", "such", "job.json").encode(), C.byref(out)) == binding.PHQ_CONFIGURATION_ERROR
+    assert global_error().startswith("Configuration error : unable to read instruction file from ")
+    assert out.value is None
+
+    handle = C.c_void_p(1)
+    assert lib.phq_create(b"{ not json", -1, C.byref(handle)) == binding.PHQ_CONFIGURATION_ERROR
+    assert global_error().startswith("Configuration error : ")
+    assert handle.value is None
+
+    tiles = (binding.Tile * 1)()
+    assert lib.phq_pack(None, 0, 0, None, None, None, tiles) == binding.PHQ_INTERNAL_ERROR
+    assert global_error() == "Internal error : null handle"
+
+    assert lib.phq_create(job, -1, C.byref(handle)) == binding.PHQ_OK
+    try:
+        assert lib.phq_tag_record_bytes(handle, None) == binding.PHQ_INTERNAL_ERROR
+        assert lib.phq_last_error(handle).decode() == "Internal error : illegal argument"
+    finally:
+        lib.phq_destroy(handle)
