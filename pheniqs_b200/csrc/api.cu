@@ -53,10 +53,20 @@ inline int pack_workers(int64_t n_reads) {
     return workers < 1 ? 1 : workers;
 }
 
+/* device memory of T, freed with its owner; the owner makes the device current before it goes (destroy) */
 template < class T > struct DeviceBuffer {
     T* pointer;
     size_t capacity;
     DeviceBuffer() : pointer(NULL), capacity(0) {}
+    DeviceBuffer(const DeviceBuffer&) = delete;
+    DeviceBuffer& operator=(const DeviceBuffer&) = delete;
+    DeviceBuffer(DeviceBuffer&& other) noexcept : pointer(other.pointer), capacity(other.capacity) { other.pointer = NULL; other.capacity = 0; }
+    DeviceBuffer& operator=(DeviceBuffer&& other) noexcept {
+        if(this != &other) { release(); pointer = other.pointer; capacity = other.capacity; other.pointer = NULL; other.capacity = 0; }
+        return *this;
+    }
+    ~DeviceBuffer() { release(); }
+    /* grow only: staging buffers keep their memory from call to call */
     void reserve(size_t count) {
         if(count > capacity) {
             release();
@@ -64,9 +74,35 @@ template < class T > struct DeviceBuffer {
             capacity = count;
         }
     }
+    /* the whole table, in memory allocated at its size (at least `minimum` elements): nothing stale lies past its end */
+    void upload(const std::vector< T >& table, size_t minimum = 0) {
+        release();
+        reserve(table.size() > minimum ? table.size() : minimum);
+        PHQ_CUDA(cudaMemcpy(pointer, table.data(), table.size() * sizeof(T), cudaMemcpyHostToDevice));
+    }
+    /* no CUDA call on an empty buffer: a host-only handle never touches the runtime */
     void release() {
         if(pointer != NULL) { cudaFree(pointer); pointer = NULL; capacity = 0; }
     }
+};
+
+/* one 16-byte record of a combinatorial codec blob (pamld_grid_kernel) */
+struct GridCell { uint32_t a, b, c, d; };
+
+/*  The device tables of one decoder and what their builders derive. Each builder resets its own part and fills it
+    where its kernel applies; an empty buffer (NULL) means the kernel does not run for this decoder. */
+struct DecoderTables {
+    DeviceBuffer< BarcodeEntry > barcodes;      /* padded to whole WHITELIST_CHUNK groups with zero entries (prior 0) */
+    DeviceBuffer< LongBarcodeEntry > long_barcodes;     /* decoders of more than LONG_NUCLEOTIDES (kernels.cuh) instead of `barcodes` */
+    DeviceBuffer< FastEntry > fast;             /* f32 form of the barcode table for the prefilter scans */
+    DeviceBuffer< GridCell > grid;              /* combinatorial codec blob (kernels.cuh) */
+    int32_t grid_a = 0, grid_b = 0, grid_entries = 0, grid_split = 0, grid_dense = 0, grid_uniform = 0;
+    DeviceBuffer< unsigned char > whitelist;    /* chunked whitelist blob (kernels.cuh) */
+    int32_t whitelist_chunks = 0;
+    double prior_maximum = 0;
+    DeviceBuffer< MddSlot > mdd;                /* MDD lookup tables (kernels.cuh), empty where the scan kernel is used */
+    int32_t mdd_first[PHQ_MAX_SEGMENTS + 1] = {}, mdd_mask[PHQ_MAX_SEGMENTS + 1] = {}, mdd_slots = 0;    /* where `mdd` holds tables: first slot and mask of every table, total slots */
+    DeviceBuffer< uint8_t > barcode_code;       /* tag synthesis: [(N + 1)][L] BAM codes, row 0 undetermined */
 };
 
 /* device staging of one in-flight sub-batch of phq_decode_batch */
@@ -84,6 +120,11 @@ struct StagingSlot {
     std::vector< DeviceBuffer< long long > > raw_offset;
     DeviceBuffer< uint8_t > aux;                /* tag synthesis: auxiliary records and their lengths */
     DeviceBuffer< int32_t > aux_length;
+    StagingSlot() : stream(NULL), done(NULL) {}
+    ~StagingSlot() {
+        if(done != NULL) { cudaEventDestroy(done); }
+        if(stream != NULL) { cudaStreamDestroy(stream); }
+    }
 };
 
 constexpr int STAGING_SLOTS = 3;
@@ -97,32 +138,21 @@ struct phq_handle {
     std::vector< DecoderSpec > chain;
     std::vector< DecoderParams > params;
     std::vector< std::vector< ScratchSegment > > scratch;
-    std::vector< BarcodeEntry* > device_barcodes;
-    std::vector< LongBarcodeEntry* > device_long;   /* the table of decoders of more than LONG_NUCLEOTIDES (kernels.cuh), NULL elsewhere */
-    std::vector< MddSlot* > device_mdd;        /* MDD lookup tables (kernels.cuh), NULL where the scan kernel is used */
-    std::vector< std::vector< int32_t > > mdd_shape;    /* per decoder: first slot and mask of every table, total slots */
-    std::vector< uint8_t* > device_barcode_code;   /* tag synthesis: [(N + 1)][L] BAM codes per coded decoder, row 0 undetermined */
-    uint8_t* device_read_group_text;            /* tag synthesis: read group IDs of the sample decoder */
-    int32_t* device_read_group_offset;
+    std::vector< DecoderTables > tables;        /* per decoder */
+    DeviceBuffer< uint8_t > device_read_group_text;     /* tag synthesis: read group IDs of the sample decoder */
+    DeviceBuffer< int32_t > device_read_group_offset;
     int32_t read_group_longest;
     bool tags_ready;
-    std::vector< unsigned char* > device_whitelist;    /* chunked whitelist blobs (kernels.cuh), NULL where not applicable */
-    std::vector< int32_t > whitelist_chunks;
-    std::vector< double > prior_maximum;
-    std::vector< FastEntry* > device_fast;     /* f32 form of the barcode tables for the prefilter scans, NULL where not applicable */
-    float* device_phred32;                      /* f32 mismatch ratios */
+    DeviceBuffer< float > device_phred32;       /* f32 mismatch ratios */
     bool fast_enabled;                          /* PHQ_DISABLE_FAST=1 keeps every PAMLD decoder on the exact scans */
-    std::vector< void* > device_grid;          /* combinatorial codec blobs (kernels.cuh), NULL where not applicable */
-    std::vector< int32_t > grid_shape;         /* per decoder: grid_a, grid_b, grid_entries, grid_split, grid_dense, grid_uniform */
-    double* device_phred;
-    unsigned char* device_accumulators;
+    DeviceBuffer< double > device_phred;
+    DeviceBuffer< unsigned char > device_accumulators;
     std::vector< int64_t > offset_u64;
     std::vector< int64_t > offset_f64;
     int64_t n_u64;
     int64_t n_f64;
     LaunchGeometry geometry;
     StagingSlot slot[STAGING_SLOTS];
-    bool slots_ready;
     DeviceBuffer< unsigned char > tie_list;  /* tie queue of the device path (one batch in flight per handle) */
     cudaEvent_t timing_start;
     cudaEvent_t timing_stop;
@@ -133,8 +163,7 @@ struct phq_handle {
     bool collected;                         /* the tables hold the sums of all ranks (phq_collect): no decode / collect until reset */
     std::string error;
 
-    phq_handle() : device(0), device_phred32(NULL), fast_enabled(true), device_read_group_text(NULL), device_read_group_offset(NULL), read_group_longest(0), tags_ready(false),
-        device_phred(NULL), device_accumulators(NULL), n_u64(0), n_f64(0), slots_ready(false),
+    phq_handle() : device(0), read_group_longest(0), tags_ready(false), fast_enabled(true), n_u64(0), n_f64(0),
         timing_start(NULL), timing_stop(NULL), timing_stream(NULL), timing_valid(false), kernel_launches(0), sub_batch_reads(SUB_BATCH_READS), collected(false) {
         /* PHQ_SUB_BATCH_READS: smaller sub-batches (tests exercise the boundaries with small inputs) */
         const char* const value(getenv("PHQ_SUB_BATCH_READS"));
@@ -142,9 +171,13 @@ struct phq_handle {
         const char* const disable(getenv("PHQ_DISABLE_FAST"));
         if(disable != NULL && atoi(disable) > 0) { fast_enabled = false; }
     }
+    ~phq_handle() {
+        if(timing_start != NULL) { cudaEventDestroy(timing_start); }
+        if(timing_stop != NULL) { cudaEventDestroy(timing_stop); }
+    }
 
-    unsigned long long* u64_plane() const { return reinterpret_cast< unsigned long long* >(device_accumulators); }
-    double* f64_plane() const { return reinterpret_cast< double* >(device_accumulators + n_u64 * 8); }
+    unsigned long long* u64_plane() const { return reinterpret_cast< unsigned long long* >(device_accumulators.pointer); }
+    double* f64_plane() const { return reinterpret_cast< double* >(device_accumulators.pointer + n_u64 * 8); }
     unsigned long long* totals() const { return u64_plane() + n_u64 - 4; }
     unsigned long long* diagnostics() const { return u64_plane() + n_u64 - 2; }
 };
@@ -198,23 +231,24 @@ void upload_barcodes(phq_handle* h, size_t k) {
             e.prior = d.concentration[b];
             table[b] = e;
         }
-        PHQ_CUDA(cudaMemcpy(h->device_long[k], table.data(), table.size() * sizeof(LongBarcodeEntry), cudaMemcpyHostToDevice));
+        h->tables[k].long_barcodes.upload(table);
         return;
     }
-    std::vector< BarcodeEntry > table(static_cast< size_t >(d.barcode_cardinality));
+    /* padded to whole whitelist groups with zero entries (prior 0): pamld_whitelist_kernel may look a padding barcode up */
+    std::vector< BarcodeEntry > table((static_cast< size_t >(d.barcode_cardinality) + WHITELIST_CHUNK - 1) / WHITELIST_CHUNK * WHITELIST_CHUNK);
     for(int32_t b(0); b < d.barcode_cardinality; ++b) {
         BarcodeEntry e;
         barcode_planes(d, b, 0, d.nucleotide_cardinality, e.lo, e.hi);
         e.prior = d.concentration[b];
         table[b] = e;
     }
-    PHQ_CUDA(cudaMemcpy(h->device_barcodes[k], table.data(), table.size() * sizeof(BarcodeEntry), cudaMemcpyHostToDevice));
+    h->tables[k].barcodes.upload(table);
 }
 
 /* the barcode table in the form the f32 prefilter scans read (pamld_fast_kernel) */
 void upload_fast(phq_handle* h, size_t k) {
     const DecoderSpec& d(h->chain[k]);
-    if(h->device_fast[k] != NULL) { cudaFree(h->device_fast[k]); h->device_fast[k] = NULL; }
+    h->tables[k].fast.release();
     /* no prefilter for long decoders: its f32 error bound is argued for at most 32 positions, and 4^-64 is below the
        smallest normal float */
     if(d.algorithm != PHQ_PAMLD || !h->fast_enabled || d.nucleotide_cardinality > LONG_NUCLEOTIDES) { return; }
@@ -226,8 +260,7 @@ void upload_fast(phq_handle* h, size_t k) {
         e.prior = static_cast< float >(d.concentration[b]);
         table[b] = e;
     }
-    PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_fast[k]), (table.size() ? table.size() : 1) * sizeof(FastEntry)));
-    PHQ_CUDA(cudaMemcpy(h->device_fast[k], table.data(), table.size() * sizeof(FastEntry), cudaMemcpyHostToDevice));
+    h->tables[k].fast.upload(table, 1);
 }
 
 /*  Combinatorial codecs (C1: 12 distinct i7 words x 8 distinct i5 words = 96 barcodes): group the barcodes
@@ -236,8 +269,9 @@ void upload_fast(phq_handle* h, size_t k) {
     segments, a supported shape, and far fewer distinct words than barcodes. */
 void upload_grid(phq_handle* h, size_t k) {
     const DecoderSpec& d(h->chain[k]);
-    if(h->device_grid[k] != NULL) { cudaFree(h->device_grid[k]); h->device_grid[k] = NULL; }
-    for(int i(0); i < 6; ++i) { h->grid_shape[k * 6 + i] = 0; }
+    DecoderTables& tables(h->tables[k]);
+    tables.grid.release();
+    tables.grid_a = tables.grid_b = tables.grid_entries = tables.grid_split = tables.grid_dense = tables.grid_uniform = 0;
     if(d.algorithm != PHQ_PAMLD || d.segment_cardinality < 2) { return; }
     const int32_t split(d.segment_length[0]);
     const int32_t L(d.nucleotide_cardinality);
@@ -261,7 +295,6 @@ void upload_grid(phq_handle* h, size_t k) {
     }
     const size_t KA(by_prefix.size()), KB(suffix_word.size());
     if((KA + KB) * 2 > static_cast< size_t >(d.barcode_cardinality) || KB > 64) { return; }
-    struct Cell { uint32_t a, b, c, d; };
     /* dense form when the codec fills most of the KA x KB grid: every A word gets KBP consecutive entries in B
        word order, absent combinations carry prior 0 (pamld_grid_kernel, KBP > 0) */
     /* separable form: the full KA x KB grid under one prior (the default of a multiplexed run before prior
@@ -271,34 +304,34 @@ void upload_grid(phq_handle* h, size_t k) {
     const size_t KBP(uniform ? KB : (KB <= 8 ? 8 : 16));
     const bool shape_dense((split == 8 && L == 16) || (split == 10 && L == 20));
     const bool dense(uniform || (shape_dense && KB <= 16 && static_cast< size_t >(d.barcode_cardinality) * 10 >= KA * KBP * 6));
-    std::vector< Cell > blob(KA + (dense ? KBP : KB));
-    std::vector< Cell > entries;
+    std::vector< GridCell > blob(KA + (dense ? KBP : KB));
+    std::vector< GridCell > entries;
     size_t at(0);
     for(const auto& run : by_prefix) {
-        Cell header;
+        GridCell header;
         header.a = run.first.first; header.b = run.first.second;
         header.c = static_cast< uint32_t >(entries.size());
         if(dense) {
-            Cell none;
+            GridCell none;
             none.a = 0; none.b = 0; none.c = 0; none.d = 0;
             const size_t first(entries.size());
             entries.resize(first + KBP, none);
             for(int32_t b : run.second) {
-                Cell& e(entries[first + static_cast< size_t >(suffix_of[b])]);
+                GridCell& e(entries[first + static_cast< size_t >(suffix_of[b])]);
                 e.a = static_cast< uint32_t >(suffix_of[b]) * 256u;
                 e.b = static_cast< uint32_t >(b);
                 memcpy(&e.c, &d.concentration[b], sizeof(double));
             }
         } else {
             for(int32_t b : run.second) {
-                Cell e;
+                GridCell e;
                 e.a = static_cast< uint32_t >(suffix_of[b]) * 256u;
                 e.b = static_cast< uint32_t >(b);
                 memcpy(&e.c, &d.concentration[b], sizeof(double));
                 entries.push_back(e);
             }
             while(entries.size() % 4 != 0) {        /* pad the run with prior 0: the product is 0 and never wins */
-                Cell e;
+                GridCell e;
                 e.a = 0; e.b = 0; e.c = 0; e.d = 0;
                 entries.push_back(e);
             }
@@ -307,29 +340,29 @@ void upload_grid(phq_handle* h, size_t k) {
         blob[at++] = header;
     }
     for(size_t i(0); i < (dense ? KBP : KB); ++i) {
-        Cell w;
+        GridCell w;
         w.a = i < KB ? suffix_word[i].first : 0u; w.b = i < KB ? suffix_word[i].second : 0u; w.c = 0; w.d = 0;
         blob[at++] = w;
     }
     blob.insert(blob.end(), entries.begin(), entries.end());
     if(blob.size() * 16 > 64 * 1024) { return; }
-    PHQ_CUDA(cudaMalloc(&h->device_grid[k], blob.size() * 16));
-    PHQ_CUDA(cudaMemcpy(h->device_grid[k], blob.data(), blob.size() * 16, cudaMemcpyHostToDevice));
-    h->grid_shape[k * 6 + 0] = static_cast< int32_t >(KA);
-    h->grid_shape[k * 6 + 1] = static_cast< int32_t >(dense ? KBP : KB);
-    h->grid_shape[k * 6 + 2] = static_cast< int32_t >(entries.size());
-    h->grid_shape[k * 6 + 3] = split;
-    h->grid_shape[k * 6 + 4] = dense ? static_cast< int32_t >(KBP) : 0;
-    h->grid_shape[k * 6 + 5] = uniform ? 1 : 0;
+    tables.grid.upload(blob);
+    tables.grid_a = static_cast< int32_t >(KA);
+    tables.grid_b = static_cast< int32_t >(dense ? KBP : KB);
+    tables.grid_entries = static_cast< int32_t >(entries.size());
+    tables.grid_split = split;
+    tables.grid_dense = dense ? static_cast< int32_t >(KBP) : 0;
+    tables.grid_uniform = uniform ? 1 : 0;
 }
 
 /*  Large single-word codecs (a cellular whitelist): the chunked blob pamld_whitelist_kernel streams — per chunk of
     WHITELIST_CHUNK barcodes the equality planes of its blocks of 32, the barcode words and the priors (kernels.cuh). */
 void upload_whitelist(phq_handle* h, size_t k) {
     const DecoderSpec& d(h->chain[k]);
-    if(h->device_whitelist[k] != NULL) { cudaFree(h->device_whitelist[k]); h->device_whitelist[k] = NULL; }
-    h->whitelist_chunks[k] = 0;
-    h->prior_maximum[k] = 0;
+    DecoderTables& tables(h->tables[k]);
+    tables.whitelist.release();
+    tables.whitelist_chunks = 0;
+    tables.prior_maximum = 0;
     long long minimum(WHITELIST_MINIMUM_BARCODES);
     const char* const value(getenv("PHQ_WHITELIST_MINIMUM"));
     if(value != NULL && atoll(value) > 0) { minimum = atoll(value); }
@@ -354,10 +387,9 @@ void upload_whitelist(phq_handle* h, size_t k) {
             if(d.concentration[b] > largest) { largest = d.concentration[b]; }
         }
     }
-    PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_whitelist[k]), blob.size()));
-    PHQ_CUDA(cudaMemcpy(h->device_whitelist[k], blob.data(), blob.size(), cudaMemcpyHostToDevice));
-    h->whitelist_chunks[k] = static_cast< int32_t >(chunks);
-    h->prior_maximum[k] = largest;
+    tables.whitelist.upload(blob);
+    tables.whitelist_chunks = static_cast< int32_t >(chunks);
+    tables.prior_maximum = largest;
 }
 
 /*  MDD lookup tables (MddSlot, kernels.cuh). Built when the reference's scan is provably a lookup: every segment
@@ -365,8 +397,9 @@ void upload_whitelist(phq_handle* h, size_t k) {
     (metric.h:87-111), so the spheres of radius `tolerance` around the distinct words of a segment are disjoint. */
 void upload_mdd_tables(phq_handle* h, size_t k) {
     const DecoderSpec& d(h->chain[k]);
-    if(h->device_mdd[k] != NULL) { cudaFree(h->device_mdd[k]); h->device_mdd[k] = NULL; }
-    h->mdd_shape[k].clear();
+    DecoderTables& tables(h->tables[k]);
+    tables.mdd.release();
+    tables.mdd_slots = 0;
     if(d.algorithm != PHQ_MDD || d.segment_cardinality > 4 || d.barcode_cardinality > MDD_MAX_BARCODES) { return; }
     if(d.nucleotide_cardinality > LONG_NUCLEOTIDES) { return; }        /* the lookup kernel reads 32-position planes */
     const int32_t S(d.segment_cardinality);
@@ -455,7 +488,6 @@ void upload_mdd_tables(phq_handle* h, size_t k) {
         entries[S].push_back(e);
     }
     /* open addressing tables, load factor <= 1/4 (mdd_probe fetches the home slot and its neighbour up front) */
-    std::vector< int32_t > shape;
     std::vector< MddSlot > blob;
     for(int32_t t(0); t <= S; ++t) {
         size_t slots(4);
@@ -468,14 +500,21 @@ void upload_mdd_tables(phq_handle* h, size_t k) {
             while(blob[first + at].value != MDD_EMPTY) { at = (at + 1) & (slots - 1); }
             blob[first + at].key_lo = e.key_lo; blob[first + at].key_hi = static_cast< uint16_t >(e.key_hi); blob[first + at].value = static_cast< uint16_t >(e.value);
         }
-        shape.push_back(static_cast< int32_t >(first));
-        shape.push_back(static_cast< int32_t >(slots - 1));
+        tables.mdd_first[t] = static_cast< int32_t >(first);
+        tables.mdd_mask[t] = static_cast< int32_t >(slots - 1);
     }
     if(blob.size() > (1u << 20)) { return; }
-    shape.push_back(static_cast< int32_t >(blob.size()));
-    PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_mdd[k]), blob.size() * sizeof(MddSlot)));
-    PHQ_CUDA(cudaMemcpy(h->device_mdd[k], blob.data(), blob.size() * sizeof(MddSlot), cudaMemcpyHostToDevice));
-    h->mdd_shape[k] = shape;
+    tables.mdd.upload(blob);
+    tables.mdd_slots = static_cast< int32_t >(blob.size());
+}
+
+/* every device table of decoder k, from its codec and its priors */
+void build_tables(phq_handle* h, size_t k) {
+    upload_barcodes(h, k);
+    upload_fast(h, k);
+    upload_grid(h, k);
+    upload_whitelist(h, k);
+    upload_mdd_tables(h, k);
 }
 
 void refresh_params(phq_handle* h, size_t k) {
@@ -517,9 +556,10 @@ void refresh_params(phq_handle* h, size_t k) {
         }
         p.uniform_observation_probability = pow(pow(10.0, -0.1), sigma);
     }
-    p.barcodes = h->device_barcodes[k];
-    p.long_barcodes = h->device_long[k];
-    p.phred = h->device_phred;
+    const DecoderTables& tables(h->tables[k]);
+    p.barcodes = tables.barcodes.pointer;
+    p.long_barcodes = tables.long_barcodes.pointer;
+    p.phred = h->device_phred.pointer;
     p.acc_u64 = h->u64_plane() + h->offset_u64[k];
     p.acc_f64 = h->f64_plane() + h->offset_f64[k];
     p.totals = NULL;
@@ -528,22 +568,21 @@ void refresh_params(phq_handle* h, size_t k) {
         p.segment_offset[s] = d.segment_offset[s];
         p.segment_length[s] = d.segment_length[s];
     }
-    p.mdd_tables = h->device_mdd[k];
+    p.mdd_tables = tables.mdd.pointer;
     if(p.mdd_tables != NULL) {
-        const std::vector< int32_t >& shape(h->mdd_shape[k]);
-        for(int32_t t(0); t <= d.segment_cardinality; ++t) { p.mdd_first[t] = shape[2 * t]; p.mdd_mask[t] = shape[2 * t + 1]; }
-        p.mdd_slots = shape.back();
+        for(int32_t t(0); t <= d.segment_cardinality; ++t) { p.mdd_first[t] = tables.mdd_first[t]; p.mdd_mask[t] = tables.mdd_mask[t]; }
+        p.mdd_slots = tables.mdd_slots;
     }
-    p.whitelist = h->device_whitelist[k];
-    p.whitelist_chunks = h->whitelist_chunks[k];
-    p.prior_maximum = h->prior_maximum[k];
-    p.grid = h->device_grid[k];
-    p.grid_a = h->grid_shape[k * 6 + 0];
-    p.grid_b = h->grid_shape[k * 6 + 1];
-    p.grid_entries = h->grid_shape[k * 6 + 2];
-    p.grid_split = h->grid_shape[k * 6 + 3];
-    p.grid_dense = h->grid_shape[k * 6 + 4];
-    p.grid_uniform = h->grid_shape[k * 6 + 5];
+    p.whitelist = tables.whitelist.pointer;
+    p.whitelist_chunks = tables.whitelist_chunks;
+    p.prior_maximum = tables.prior_maximum;
+    p.grid = tables.grid.pointer;
+    p.grid_a = tables.grid_a;
+    p.grid_b = tables.grid_b;
+    p.grid_entries = tables.grid_entries;
+    p.grid_split = tables.grid_split;
+    p.grid_dense = tables.grid_dense;
+    p.grid_uniform = tables.grid_uniform;
     {
         /* one bit of a tie block mask per (4 << shift) scanned barcodes / grid entries: at most 32 bits */
         const int32_t scanned(p.grid != NULL ? p.grid_entries : p.barcode_cardinality);
@@ -551,11 +590,11 @@ void refresh_params(phq_handle* h, size_t k) {
         while((((scanned + 3) >> 2) + (1 << shift) - 1) >> shift > 32) { ++shift; }
         p.tie_block_shift = shift;
     }
-    /* the prefilter scan exists for the generic scan and for the separable form of the combinatorial one */
-    const bool dense_shape((p.grid_split == 8 && p.nucleotide_cardinality == 16) || (p.grid_split == 10 && p.nucleotide_cardinality == 20));
-    const bool prefilter(h->device_fast[k] != NULL && p.whitelist == NULL && (p.grid == NULL || p.grid_uniform != 0 || (p.grid_dense != 0 && dense_shape)));
-    p.fast_barcodes = prefilter ? h->device_fast[k] : NULL;
-    p.phred32 = h->device_phred32;
+    /* the prefilter scan exists for the generic scan and for the dense forms of the combinatorial one (upload_grid
+       builds a dense grid only for the separable form and the 8 + 8 and 10 + 10 shapes) */
+    const bool prefilter(tables.fast.pointer != NULL && p.whitelist == NULL && (p.grid == NULL || p.grid_dense != 0));
+    p.fast_barcodes = prefilter ? tables.fast.pointer : NULL;
+    p.phred32 = h->device_phred32.pointer;
     p.fast_uniform_prior = 0.0f;
     if(prefilter && d.barcode_cardinality > 0) {
         bool uniform(true);
@@ -566,40 +605,7 @@ void refresh_params(phq_handle* h, size_t k) {
 
 void destroy(phq_handle* h) {
     if(h == NULL) { return; }
-    if(h->device < 0) { delete h; return; }
-    cudaSetDevice(h->device);
-    for(auto* p : h->device_barcodes) { if(p != NULL) { cudaFree(p); } }
-    for(auto* p : h->device_long) { if(p != NULL) { cudaFree(p); } }
-    for(auto* p : h->device_grid) { if(p != NULL) { cudaFree(p); } }
-    for(auto* p : h->device_fast) { if(p != NULL) { cudaFree(p); } }
-    if(h->device_phred32 != NULL) { cudaFree(h->device_phred32); }
-    for(auto* p : h->device_whitelist) { if(p != NULL) { cudaFree(p); } }
-    for(auto* p : h->device_barcode_code) { if(p != NULL) { cudaFree(p); } }
-    if(h->device_read_group_text != NULL) { cudaFree(h->device_read_group_text); }
-    if(h->device_read_group_offset != NULL) { cudaFree(h->device_read_group_offset); }
-    for(auto* p : h->device_mdd) { if(p != NULL) { cudaFree(p); } }
-    if(h->device_phred != NULL) { cudaFree(h->device_phred); }
-    if(h->device_accumulators != NULL) { cudaFree(h->device_accumulators); }
-    if(h->slots_ready) {
-        for(auto& s : h->slot) {
-            for(auto& b : s.bases) { b.release(); }
-            for(auto& b : s.nmask) { b.release(); }
-            for(auto& b : s.quality) { b.release(); }
-            for(auto& b : s.results) { b.release(); }
-            for(auto& b : s.raw_sequence) { b.release(); }
-            for(auto& b : s.raw_quality) { b.release(); }
-            for(auto& b : s.raw_offset) { b.release(); }
-            s.qcfail.release();
-            s.aux.release();
-            s.aux_length.release();
-            s.tie_list.release();
-            cudaEventDestroy(s.done);
-            cudaStreamDestroy(s.stream);
-        }
-    }
-    h->tie_list.release();
-    if(h->timing_start != NULL) { cudaEventDestroy(h->timing_start); }
-    if(h->timing_stop != NULL) { cudaEventDestroy(h->timing_stop); }
+    if(h->device >= 0) { cudaSetDevice(h->device); }       /* its buffers, streams and events go on its own device */
     delete h;
 }
 
@@ -671,15 +677,14 @@ void launch_chain(phq_handle* h, int64_t n_reads, const phq_tile* tiles, uint8_t
     }
 }
 
+/* a retry after a failure creates only what the failed call did not */
 void ensure_slots(phq_handle* h) {
-    if(h->slots_ready) { return; }
     const size_t n(h->chain.size());
     for(auto& s : h->slot) {
-        PHQ_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-        PHQ_CUDA(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
+        if(s.stream == NULL) { PHQ_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking)); }
+        if(s.done == NULL) { PHQ_CUDA(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming)); }
         s.bases.resize(n); s.nmask.resize(n); s.quality.resize(n); s.results.resize(n);
     }
-    h->slots_ready = true;
 }
 
 /*  The status of the exception in flight; its message goes where phq_last_error finds it: on the handle, or in the
@@ -873,16 +878,7 @@ int phq_create(const char* compiled_job_json, int device, phq_handle** handle) {
         h->geometry.shared_memory_per_block_optin = prop.sharedMemPerBlockOptin;
         const size_t n(chain.size());
         h->params.resize(n);
-        h->device_barcodes.assign(n, NULL);
-        h->device_long.assign(n, NULL);
-        h->device_grid.assign(n, NULL);
-        h->device_fast.assign(n, NULL);
-        h->device_whitelist.assign(n, NULL);
-        h->whitelist_chunks.assign(n, 0);
-        h->prior_maximum.assign(n, 0.0);
-        h->device_mdd.assign(n, NULL);
-        h->mdd_shape.assign(n, std::vector< int32_t >());
-        h->grid_shape.assign(n * 6, 0);
+        h->tables.resize(n);
         h->scratch.resize(n);
         h->offset_u64.resize(n);
         h->offset_f64.resize(n);
@@ -896,37 +892,21 @@ int phq_create(const char* compiled_job_json, int device, phq_handle** handle) {
         }
         h->n_u64 = at_u + 4;        /* + totals count, pf_count + diagnostics exact path, threshold band */
         h->n_f64 = at_f;
-        PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_accumulators), static_cast< size_t >(h->n_u64 + h->n_f64) * 8));
-        PHQ_CUDA(cudaMemset(h->device_accumulators, 0, static_cast< size_t >(h->n_u64 + h->n_f64) * 8));
+        h->device_accumulators.reserve(static_cast< size_t >(h->n_u64 + h->n_f64) * 8);
+        PHQ_CUDA(cudaMemset(h->device_accumulators.pointer, 0, static_cast< size_t >(h->n_u64 + h->n_f64) * 8));
 
         std::vector< double > phred;
         double uniform_quality, base;
         assemble_phred(phred, uniform_quality, base);
-        PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_phred), phred.size() * sizeof(double)));
-        PHQ_CUDA(cudaMemcpy(h->device_phred, phred.data(), phred.size() * sizeof(double), cudaMemcpyHostToDevice));
+        h->device_phred.upload(phred);
         {
-            float ratio32[128];
+            std::vector< float > ratio32(128);
             for(int q(0); q < 128; ++q) { ratio32[q] = static_cast< float >(phred[PHRED_MISMATCH_RATIO + q]); }
-            PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_phred32), sizeof(ratio32)));
-            PHQ_CUDA(cudaMemcpy(h->device_phred32, ratio32, sizeof(ratio32), cudaMemcpyHostToDevice));
+            h->device_phred32.upload(ratio32);
         }
 
         for(size_t k(0); k < n; ++k) {
-            if(chain[k].tiled()) {
-                if(chain[k].nucleotide_cardinality > LONG_NUCLEOTIDES) {
-                    PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_long[k]), static_cast< size_t >(chain[k].barcode_cardinality) * sizeof(LongBarcodeEntry)));
-                } else {
-                    /* padded to whole whitelist groups with zero entries (prior 0): pamld_whitelist_kernel may look a padding barcode up */
-                    const size_t padded((static_cast< size_t >(chain[k].barcode_cardinality) + WHITELIST_CHUNK - 1) / WHITELIST_CHUNK * WHITELIST_CHUNK);
-                    PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_barcodes[k]), padded * sizeof(BarcodeEntry)));
-                    PHQ_CUDA(cudaMemset(h->device_barcodes[k], 0, padded * sizeof(BarcodeEntry)));
-                }
-                upload_barcodes(h, k);
-                upload_fast(h, k);
-                upload_grid(h, k);
-                upload_whitelist(h, k);
-                upload_mdd_tables(h, k);
-            }
+            if(chain[k].tiled()) { build_tables(h, k); }
             refresh_params(h, k);
         }
         PHQ_CUDA(cudaEventCreate(&h->timing_start));
@@ -1298,17 +1278,14 @@ int32_t host_read_group_longest(const phq_handle* h) {
 /* device tables of the tag kernel: barcode codes by index (row 0 = undetermined) and the read group IDs */
 void ensure_tags(phq_handle* h) {
     if(h->tags_ready) { return; }
-    const size_t n(h->chain.size());
-    h->device_barcode_code.assign(n, NULL);
     const char* name[3] = { "sample", "molecular", "cellular" };
-    for(size_t k(0); k < n; ++k) {
+    for(size_t k(0); k < h->chain.size(); ++k) {
         const DecoderSpec& d(h->chain[k]);
         if(!d.tiled()) { continue; }
         const size_t L(static_cast< size_t >(d.nucleotide_cardinality));
         std::vector< uint8_t > table((static_cast< size_t >(d.barcode_cardinality) + 1) * L, 0);
         memcpy(table.data() + L, d.barcode.data(), static_cast< size_t >(d.barcode_cardinality) * L);
-        PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_barcode_code[k]), table.size() ? table.size() : 1));
-        PHQ_CUDA(cudaMemcpy(h->device_barcode_code[k], table.data(), table.size(), cudaMemcpyHostToDevice));
+        h->tables[k].barcode_code.upload(table, 1);
         if(d.topic == PHQ_SAMPLE) {
             /* decode_tag_id_by_index (classifier.h): the ID of the undetermined element, then of every barcode by index */
             const Json* element(h->job.find(name[0]));
@@ -1323,10 +1300,8 @@ void ensure_tags(phq_handle* h) {
             push(element != NULL ? element->find("undetermined") : NULL);
             const Json* codec(element != NULL ? element->find("codec") : NULL);
             for(const auto& key : d.barcode_key) { push(codec != NULL ? codec->find(key) : NULL); }
-            PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_read_group_text), text.size() ? text.size() : 1));
-            PHQ_CUDA(cudaMemcpy(h->device_read_group_text, text.data(), text.size(), cudaMemcpyHostToDevice));
-            PHQ_CUDA(cudaMalloc(reinterpret_cast< void** >(&h->device_read_group_offset), offset.size() * sizeof(int32_t)));
-            PHQ_CUDA(cudaMemcpy(h->device_read_group_offset, offset.data(), offset.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+            h->device_read_group_text.upload(std::vector< uint8_t >(text.begin(), text.end()), 1);
+            h->device_read_group_offset.upload(offset);
         }
     }
     h->tags_ready = true;
@@ -1434,8 +1409,8 @@ int decode_raw(phq_handle* handle, int64_t n_reads, int32_t n_input_segments, co
             plan.phred_offset = phred_offset;
             plan.bam_input = bam_input ? 1 : 0;
             plan.stride = aux_stride;
-            plan.read_group_text = h->device_read_group_text;
-            plan.read_group_offset = h->device_read_group_offset;
+            plan.read_group_text = h->device_read_group_text.pointer;
+            plan.read_group_offset = h->device_read_group_offset.pointer;
             memcpy(plan.input, view, sizeof(view));
             for(size_t k(0); k < n_decoders; ++k) {
                 const DecoderSpec& d(h->chain[k]);
@@ -1449,7 +1424,7 @@ int decode_raw(phq_handle* handle, int64_t n_reads, int32_t n_input_segments, co
                 for(int32_t i(0); i <= d.segment_cardinality && i <= PHQ_MAX_SEGMENTS && !d.transform.empty(); ++i) { to.segment_offset[i] = d.segment_offset[i]; }
                 for(size_t i(0); i < d.transform.size(); ++i) { to.token[i] = pack_token(d.transform[i]); }
                 to.results = d.tiled() ? device_results[k] : NULL;
-                to.barcode_code = h->device_barcode_code[k];
+                to.barcode_code = h->tables[k].barcode_code.pointer;
             }
             s.aux.reserve(static_cast< size_t >(sub) * aux_stride);
             s.aux_length.reserve(static_cast< size_t >(sub));
@@ -1551,7 +1526,7 @@ int phq_totals(phq_handle* handle, uint64_t* count, uint64_t* pf_count) {
 
 int phq_accumulator_buffer(phq_handle* handle, void** device_pointer, int64_t* n_u64, int64_t* n_f64) {
     return guarded(handle, [&]() {
-        if(device_pointer != NULL) { *device_pointer = handle->device_accumulators; }
+        if(device_pointer != NULL) { *device_pointer = handle->device_accumulators.pointer; }
         if(n_u64 != NULL) { *n_u64 = handle->n_u64; }
         if(n_f64 != NULL) { *n_f64 = handle->n_f64; }
     });
@@ -1560,14 +1535,14 @@ int phq_accumulator_buffer(phq_handle* handle, void** device_pointer, int64_t* n
 int phq_reset_accumulators(phq_handle* handle) {
     return guarded(handle, [&]() {
         PHQ_CUDA(cudaDeviceSynchronize());
-        PHQ_CUDA(cudaMemset(handle->device_accumulators, 0, static_cast< size_t >(handle->n_u64 + handle->n_f64) * 8));
+        PHQ_CUDA(cudaMemset(handle->device_accumulators.pointer, 0, static_cast< size_t >(handle->n_u64 + handle->n_f64) * 8));
         handle->collected = false;
     });
 }
 
 int phq_reset_accumulators_async(phq_handle* handle, void* stream) {
     return guarded(handle, [&]() {
-        PHQ_CUDA(cudaMemsetAsync(handle->device_accumulators, 0, static_cast< size_t >(handle->n_u64 + handle->n_f64) * 8, static_cast< cudaStream_t >(stream)));
+        PHQ_CUDA(cudaMemsetAsync(handle->device_accumulators.pointer, 0, static_cast< size_t >(handle->n_u64 + handle->n_f64) * 8, static_cast< cudaStream_t >(stream)));
         handle->collected = false;
     });
 }
@@ -1622,10 +1597,7 @@ int phq_set_priors(phq_handle* handle, int decoder, double noise, const double* 
             for(int32_t i(0); i < d.barcode_cardinality; ++i) { d.concentration[i] = concentration[i]; }
         }
         PHQ_CUDA(cudaDeviceSynchronize());
-        upload_barcodes(handle, static_cast< size_t >(decoder));
-        upload_fast(handle, static_cast< size_t >(decoder));
-        upload_grid(handle, static_cast< size_t >(decoder));
-        upload_whitelist(handle, static_cast< size_t >(decoder));
+        build_tables(handle, static_cast< size_t >(decoder));
         refresh_params(handle, static_cast< size_t >(decoder));
     });
 }

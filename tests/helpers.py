@@ -69,6 +69,29 @@ def random_job(rng, algorithm="pamld", segments=(8,), n_barcodes=24, reverse=Fal
     return decoder
 
 
+def grid_job(la, lb, ka, kb, fill, equal):
+    """A dual index PAMLD job: ka distinct first words of la nt times kb distinct second words of lb nt, each
+    combination present with probability `fill`, under equal priors or priors of 1 to 3."""
+    rng = np.random.default_rng(la * 100 + ka)
+    letters = np.frombuffer(b"ACGT", dtype=np.uint8)
+
+    def words(count, length):
+        out = []
+        while len(out) < count:
+            w = rng.integers(0, 4, size=length)
+            if all((w != v).sum() >= 3 for v in out):
+                out.append(w)
+        return [letters[w].tobytes().decode() for w in out]
+    first, second = words(ka, la), words(kb, lb)
+    codec = {}
+    for i, a in enumerate(first):
+        for j, b in enumerate(second):
+            if rng.random() < fill:
+                codec["@%02d_%02d" % (j, i)] = {"barcode": [a, b], "concentration": 1.0 if equal else float(rng.integers(1, 4))}
+    return {"sample": {"algorithm": "pamld", "transform": {"token": ["0:0:%d" % la, "1:0:%d" % lb]}, "codec": codec, "noise": 0.04,
+                       "confidence threshold": 0.9, "high quality threshold": 20, "high quality distance threshold": 2}}
+
+
 def compare_pamld(got, expected_index, expected_distance, expected_confidence, label=""):
     assert np.array_equal(got["index"], expected_index), label + " barcode index"
     assert np.array_equal(got["distance"], expected_distance), label + " distance"

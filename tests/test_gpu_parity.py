@@ -4,6 +4,8 @@ Bar (BASELINE.json north_star, SURVEY.md §8d): barcode index, distance and qcfa
 PAMLD; PAMLD posterior within 1e-6 in log space (and the error probability 1 - conf within 1e-6 relative,
 floored at the 2^-53 quantum of the reference's own `1.0 - confidence`); u64 accumulators identical;
 f64 accumulators and estimated priors within 1e-9 relative."""
+import copy
+
 import numpy as np
 import pytest
 
@@ -193,26 +195,7 @@ def test_combinatorial_codecs(shape):
     """Dual-index style codecs (distinct first-segment words x distinct second-segment words) take the
     combinatorial scan kernel: sparse grids (runs not a multiple of four), dense grids with absent
     combinations, and full grids with equal priors (the separable form: KA + KB word products per read)."""
-    la, lb, ka, kb, fill, equal = shape
-    rng = np.random.default_rng(la * 100 + ka)
-    letters = np.frombuffer(b"ACGT", dtype=np.uint8)
-
-    def words(count, length):
-        out = []
-        while len(out) < count:
-            w = rng.integers(0, 4, size=length)
-            if all((w != v).sum() >= 3 for v in out):
-                out.append(w)
-        return [letters[w].tobytes().decode() for w in out]
-    first, second = words(ka, la), words(kb, lb)
-    codec = {}
-    for i, a in enumerate(first):
-        for j, b in enumerate(second):
-            if rng.random() < fill:
-                codec["@%02d_%02d" % (j, i)] = {"barcode": [a, b], "concentration": 1.0 if equal else float(rng.integers(1, 4))}
-    job = {"sample": {"algorithm": "pamld", "transform": {"token": ["0:0:%d" % la, "1:0:%d" % lb]}, "codec": codec, "noise": 0.04, "confidence threshold": 0.9,
-                      "high quality threshold": 20, "high quality distance threshold": 2}}
-    compiled = compile_job(job)
+    compiled = compile_job(helpers.grid_job(*shape))
     code, quality, offset, _ = workload.synthesize(compiled, [0], 30000, seed=8)
     check(*run_both(None, code, quality, offset, compiled=compiled))
 
@@ -311,6 +294,67 @@ def test_two_pass_prior_estimation():
     expected2 = second.decode(O.ReadBatch(code, quality, offset))
     check(chain, second, results2, flags2, expected2)
     assert not np.array_equal(results2[1]["confidence"], results[1]["confidence"])
+
+
+def priors(compiled):
+    """The sample decoder's barcode priors in index order."""
+    codec = compiled["sample"]["codec"]
+    return np.array([r["concentration"] for r in sorted(codec.values(), key=lambda r: r["index"])])
+
+
+def check_with_priors(chain, compiled, tiles, concentration, code, quality, offset, qcfail):
+    """Give the sample decoder `concentration` through set_priors, decode `tiles` again and compare with the oracle
+    under the same priors."""
+    chain.set_priors(0, compiled["sample"]["noise"], concentration)
+    job = copy.deepcopy(compiled)
+    for record in job["sample"]["codec"].values():
+        record["concentration"] = float(concentration[record["index"] - 1])
+    chain.reset()
+    results, flags = chain.decode(tiles, len(qcfail), qcfail)
+    checker = O.best_oracle(job, len(code))
+    check(chain, checker, results, flags, checker.decode(O.ReadBatch(code, quality, offset, qcfail)))
+
+
+def test_set_priors_rebuilds_the_grid_form():
+    """A full 6 + 6 grid takes the separable form and the prefilter under equal priors, the sparse form without the
+    prefilter under unequal ones, and the separable form again when equal priors come back: the grid table is
+    rebuilt at another size each time, and the prefilter table stays allocated while the sparse form gates it off."""
+    compiled = compile_job(helpers.grid_job(6, 6, 4, 5, 1.0, True))
+    n = 20000
+    code, quality, offset, _ = workload.synthesize(compiled, [0], n, seed=10)
+    qcfail = (np.random.default_rng(10).random(n) < 0.1).astype(np.uint8)
+    chain = DecoderChain(compiled, device=0)
+    tiles = chain.pack(code, quality, offset)
+    equal = priors(compiled)
+    unequal = equal * (1 + np.arange(equal.size) % 3)
+    unequal *= equal.sum() / unequal.sum()
+    assert chain.kernel_description(0).startswith("pamld_fast_grid_kernel<6, 6, 0>")
+    for concentration, separable in ((equal, True), (unequal, False), (equal, True)):
+        check_with_priors(chain, compiled, tiles, concentration, code, quality, offset, qcfail)
+        description = chain.kernel_description(0)
+        if separable:
+            assert description.startswith("pamld_fast_grid_kernel<6, 6, 0>"), description
+        else:
+            assert description.startswith("pamld_grid_kernel<6, 6, 2, 0, 0> + ") and "pamld_fast" not in description, description
+
+
+def test_set_priors_rebuilds_the_whitelist_bound(monkeypatch):
+    """The whitelist scan prunes with the largest prior as its bound: a prior raised above every other through
+    set_priors must raise the bound, or reads of that barcode are pruned away."""
+    monkeypatch.setenv("PHQ_WHITELIST_MINIMUM", "1")
+    rng = np.random.default_rng(79)
+    compiled = compile_job({"sample": helpers.random_job(rng, "pamld", (10,), 300, minimum_distance=2)})
+    n = 12000
+    code, quality, offset, _ = workload.synthesize(compiled, [0], n, seed=11)
+    qcfail = (rng.random(n) < 0.1).astype(np.uint8)
+    chain = DecoderChain(compiled, device=0)
+    tiles = chain.pack(code, quality, offset)
+    concentration = priors(compiled)
+    concentration[np.argmax(concentration)] = 0.5
+    concentration *= (1 - compiled["sample"]["noise"]) / concentration.sum()
+    assert concentration.max() > 20 * priors(compiled).max()
+    check_with_priors(chain, compiled, tiles, concentration, code, quality, offset, qcfail)
+    assert chain.kernel_description(0).startswith("pamld_whitelist_kernel")
 
 
 def test_large_batch_properties():

@@ -166,35 +166,13 @@ GRIDS = {
 }
 
 
-def grid_job(form):
-    (la, lb, ka, kb, fill, equal), _ = GRIDS[form]
-    rng = np.random.default_rng(la * 100 + ka)
-    letters = np.frombuffer(b"ACGT", dtype=np.uint8)
-
-    def words(count, length):
-        out = []
-        while len(out) < count:
-            w = rng.integers(0, 4, size=length)
-            if all((w != v).sum() >= 3 for v in out):
-                out.append(w)
-        return [letters[w].tobytes().decode() for w in out]
-    first, second = words(ka, la), words(kb, lb)
-    codec = {}
-    for i, a in enumerate(first):
-        for j, b in enumerate(second):
-            if rng.random() < fill:
-                codec["@%02d_%02d" % (j, i)] = {"barcode": [a, b], "concentration": 1.0 if equal else float(rng.integers(1, 4))}
-    return {"sample": {"algorithm": "pamld", "transform": {"token": ["0:0:%d" % la, "1:0:%d" % lb]}, "codec": codec, "noise": 0.04,
-                       "confidence threshold": 0.9, "high quality threshold": 20, "high quality distance threshold": 2}}
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("form, kind", [(f, k) for f in GRIDS for k in DISTRIBUTIONS if k in SHORT_RANGES or f != "dense_10_10"])
 def test_combinatorial_grid(form, kind, monkeypatch):
     """Dual index codecs on the combinatorial scan: the separable form, dense 8 + 8 and 10 + 10 grids (20 nt: no
     qualities above 93), a sparse grid."""
     use_the_restatement(monkeypatch, kind)
-    compiled, code, quality, offset, qcfail = reads(grid_job(form), kind, 6000, seed=47)
+    compiled, code, quality, offset, qcfail = reads(helpers.grid_job(*GRIDS[form][0]), kind, 6000, seed=47)
     state = run_both(None, code, quality, offset, qcfail, compiled=compiled)
     description = state[0].kernel_description(0)
     assert description.startswith(GRIDS[form][1]), description
